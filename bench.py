@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """PPO-update benchmark on the Humanoid shape (BASELINE.json metric/config), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* is one PPO iteration's update over one synthetic rollout: the advantage pipeline
@@ -219,12 +219,10 @@ def run_reference(args, config):
     arm.warm_up()
     t_gae, t_train, mem = arm.timed_step(1)  # also sizes the sample: epochs per step within the budget
     n_ep = max(1, min(args.epochs, args.ref_epochs, int(args.ref_budget / max(t_train, 1e-3))))
-    vals, wall = [], time.perf_counter()
-    for k in range(max(1, args.steps)):
+    vals = []
+    for k in range(args.steps):
         t_gae, t_train, mem = arm.timed_step(n_ep)
         vals.append(n_ep * arm.nb * arm.B / (t_train + t_gae * n_ep / arm.E))
-        if time.perf_counter() - wall > 180:  # whatever K is, the arm ends within a few minutes
-            break
     value = sum(vals) / len(vals)
     cb = {"value": value, "unit": "samples/s", "cores": arm.cores, "kind": arm.kind, "sample": arm.describe(t_gae, t_train, n_ep),
           "gae_GBps": 21 * arm.M / 1e9 / t_gae}
@@ -451,6 +449,34 @@ def cpu_baseline(args):
     return out
 
 
+DUMP_MAX_ELEMENTS = 4 << 20  # per dumped array (16 MB in float32): the files of one dump stay under 64 MB in all
+
+
+def dump_outputs(out_dir, agent, mem, losses):
+    """`--dump-outputs`: what the last timed step hands a caller of `PPO.calculate_advantages` + `PPO.train`, as float32
+    `out_dir/<name>.npy` — the advantages and value targets written into the rollout, the per-minibatch (actor, critic)
+    losses, and the updated parameters and Adam moments under their `state_dict` names.  An array of more than
+    DUMP_MAX_ELEMENTS values keeps a seeded sample of its rows (environments, minibatches): the same rows for the same
+    arguments, so that dumps of two builds compare file for file."""
+    import numpy as np
+    eng = agent.engine
+    named = list(agent.networks.named_parameters())
+    out = {"advantage": mem["advantage"], "current_state_value_target": mem["current_state_value_target"], "losses": losses}
+    for prefix, flat in (("param", eng.flat), ("adam_exp_avg", eng.exp_avg), ("adam_exp_avg_sq", eng.exp_avg_sq)):
+        out.update({f"{prefix}.{name}": t for name, t in eng.grads_by_name(flat, named).items()})
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in out.items():
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            rows = max(1, DUMP_MAX_ELEMENTS // (t.numel() // t.shape[0]))
+            keep = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values
+            t = t[keep.to(t.device)]
+        a = t.detach().to("cpu", torch.float32).numpy()
+        total += a.nbytes
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    assert total <= 64 << 20, f"--dump-outputs wrote {total} bytes"
+
+
 def run_b200(args, config):
     import torch.distributed as dist
 
@@ -512,6 +538,7 @@ def run_b200(args, config):
     samples_per_step = E * nb * GB
 
     def step_device(i):
+        """One step; returns its losses and the rollout memory it wrote the advantages and value targets into."""
         mem = pkg.RolloutMemory(dict(d), (n_envs, T))
         algo.calculate_advantages(mem)
         fields = {"current_state": mem["current_state"].reshape(M_local, OBS_DIM), "action": mem["action"].reshape(M_local, ACT_DIM),
@@ -519,8 +546,9 @@ def run_b200(args, config):
                   "current_state_value_target": mem["current_state_value_target"].reshape(M_local)}
         if world > 1:
             fields = D.share_rollout(eng, fields)
-        return eng.train(fields["current_state"], fields["action"], fields["action_log_prob"], fields["advantage"],
-                         fields["current_state_value_target"], perms_dev[i], GB, hp)
+        losses = eng.train(fields["current_state"], fields["action"], fields["action_log_prob"], fields["advantage"],
+                           fields["current_state_value_target"], perms_dev[i], GB, hp)
+        return losses, mem
 
     def barrier():
         if world > 1:
@@ -538,7 +566,7 @@ def run_b200(args, config):
     barrier()
     ev0.record()
     for k in range(args.steps):
-        losses = step_device(args.warmup + k)
+        losses, last_mem = step_device(args.warmup + k)
     ev1.record()
     barrier()
     launches = lib.b200ppo_launch_count() - launches0
@@ -550,6 +578,8 @@ def run_b200(args, config):
         ms = float(tmax.item())
     value = args.steps * samples_per_step / (ms * 1e-3)
     final_losses = losses[-1].tolist()
+    if args.dump_outputs and rank == 0:  # before the measurements below move the parameters on
+        dump_outputs(args.dump_outputs, agent, last_mem, losses)
 
     # ---- e2e through the C ABI with host buffers (single GPU: the host entry point is per-rank) --------------
     e2e = None
@@ -832,7 +862,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline sample")
     ap.add_argument("--no-variants", action="store_true", help="skip the secondary (precision, minibatch) settings")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the host-buffer end-to-end measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (advantages, value targets, losses, updated parameters and Adam "
+                         "moments) as float32 DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -7,7 +7,7 @@ Round-1 measurement (fraction of the 6547 GB/s copy peak; random permutation / i
   two bulk copies in flight per lane (removed)     0.536 / 0.703   (halves the resident warps)
 """
 import sys, torch, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 import mujoco_reinforcement_learning_b200 as pkg
 m=4096*128; dev="cuda"

@@ -2,8 +2,8 @@
 
 B200PPO_DEBUG_DGRAD=1 traces the dgrad epilogue instead of the forward one, B200PPO_DEBUG_RELU=1 drops the MUFU work,
 B200PPO_DEBUG_TWICE=1 launches the problem twice in one group (actor + critic)."""
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from mujoco_reinforcement_learning_b200 import _lib
 lib = _lib.load()
 shapes = [(32768, 256, 256), (32768, 256, 376)]

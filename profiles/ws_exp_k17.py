@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from mujoco_reinforcement_learning_b200 import _lib
 lib = _lib.load()
 for (M, N, K) in [(65536, 128, 17)]:
