@@ -249,9 +249,9 @@ int b200ppo_profile_begin(b200ppo_ctx* ctx);
 int b200ppo_profile_end(b200ppo_ctx* ctx, double ms_out[B200PPO_PROF_CLASSES], int64_t launches_out[B200PPO_PROF_CLASSES]);
 /* Test hook for the tcgen05 GEMM kernel: C[M,N] (fp32) = A * B^T with operands rounded to bf16.  A is [M,K]
  * (a_mn_major = 0) or [K,M] (a_mn_major = 1); B is [N,K] or [K,N]; bn in {64,128,192,256}, or -1 for the
- * persistent weights-stationary kernel (K-major A, N <= 256, split_k = 1); -2: its forward (tanh) epilogue with a
- * clock64 timeline on stderr; -3: forward epilogue, C = float(bf16(tanh(A B^T))); -4: dgrad epilogue, C holds the
- * activation operand h on entry and float(bf16(A B^T (1 - bf16(h)^2))) on return; split_k >= 1.
+ * persistent weights-stationary kernel (K-major A, N <= 256, split_k = 1); -3: its forward epilogue,
+ * C = float(bf16(tanh(A B^T))); -4: its dgrad epilogue, C holds the activation operand h on entry and
+ * float(bf16(A B^T (1 - bf16(h)^2))) on return; split_k >= 1.
  * Allocates temporaries and synchronises `stream`. */
 int b200ppo_debug_tc_gemm(const float* A, const float* B, float* C, int32_t M, int32_t N, int32_t K, int32_t a_mn_major,
                           int32_t b_mn_major, int32_t bn, int32_t split_k, b200ppo_stream stream);
@@ -271,7 +271,7 @@ int b200ppo_rollout_step(b200ppo_ctx* ctx, const float* params, const float* obs
  * handed to tcgen05.  3 (default): three bf16 terms, six products per fp32 product — 24-bit operands, north_star's 1e-5
  * variant.  2: two fp16 terms of the value scaled by a power of two taken from the tensor's largest magnitude, three
  * products — 22-bit operands, about 1.3x faster; gradients stay within 1e-5 of their tensor's scale, sums that cancel
- * 1000 : 1 do not (DESIGN.md §3.3).  Env B200PPO_SPLIT_TERMS overrides. */
+ * 1000 : 1 do not (DESIGN.md §3.3). */
 int b200ppo_set_fp32_terms(b200ppo_ctx* ctx, int32_t terms);
 
 /* Test hook for the fp32-tolerance tensor-core GEMM (csrc/gemm_split.cu: three bf16 terms per operand value, six products):

@@ -563,9 +563,8 @@ static int backward_nets_bf16(b200ppo_ctx* ctx, const __nv_bfloat16* xb, int64_t
   // N tile: the width that wastes the least padded MMA work over all problems (N = in+1 is 257 / 377 for 256 / 376
   // inputs: 192-wide tiles cover both in two tiles where 128-wide ones need three); split-K: as many splits as fill
   // ONE wave of resident CTAs — one CTA more than a wave would double the kernel's duration.
-  static const char* wg_mode = getenv("B200PPO_WGRAD");  // profiling switch: "tile" keeps the one-tile kernel
   const int n_problems = ctx->net[0].d.n_layers + ctx->net[1].d.n_layers;
-  if (B >= 2048 && n_problems <= kMaxTcProblems && !(wg_mode != nullptr && wg_mode[0] == 't')) {
+  if (B >= 2048 && n_problems <= kMaxTcProblems) {
     // CTA pairs: 256 x 256 output blocks, bias gradient from a ones-tile MMA (tc_wgrad.cu)
     TcGroup g{};
     for (int n = 0; n < 2; ++n) {
@@ -1297,10 +1296,9 @@ extern "C" B2_EXPORT int b200ppo_train(b200ppo_ctx* ctx, float* params, float* e
                                  ctx->sh_adv + r0, ctx->sh_tgt + r0, lb, hp, red_losses, &split, &loss_ctas, st));
         const LossCombine lc = make_loss_combine(ctx, params, loss_ctas, lb, hp, red_losses);
         // the sum of this rank's split-K partials into its exchange buffer happens inside the optimizer kernel (one
-        // element per thread); B200PPO_P2P_FUSED_REDUCE=0 keeps the separate launch in front of it
-        static const bool fused_env = []() { const char* e = getenv("B200PPO_P2P_FUSED_REDUCE"); return !(e != nullptr && e[0] == '0'); }();
+        // element per thread); a small grid or no loss partials keep the separate launch in front of it
         const int agrid = adam_cast_grid(ctx->n_params);
-        const bool fused = fused_env && loss_ctas > 0 && int64_t(agrid) * 256 >= ctx->n_params / 4;
+        const bool fused = loss_ctas > 0 && int64_t(agrid) * 256 >= ctx->n_params / 4;
         if (!fused) PROF(ctx, B200PPO_PROF_OTHER, st, launch_reduce_partials(ctx->gpart, split, ctx->n_params, ctx->n_params, xb, st, &lc));
         PeerSrc ps{};
         ps.world = ctx->world; ps.rank = ctx->rank; ps.seq = seq; ps.err = ctx->err_flag; ps.losses_out = loss_slot;

@@ -12,8 +12,6 @@
 
 #include <algorithm>
 
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace b200ppo {
@@ -218,8 +216,7 @@ int launch_gather_chunked(const int64_t* idx, int64_t count, int64_t n_rows, int
   if (count == 0) return B200PPO_OK;
   const bool vec = (obs_dim % 4 == 0) && aligned16(obs) && aligned16(obs_o);
   const size_t tma_smem = size_t(32) * obs_dim * 4;
-  static const char* mode = getenv("B200PPO_GATHER");  // profiles/gather_variants.py: "ldg" forces the load/store kernel
-  if (vec && tma_smem <= 56 * 1024 && count >= 4096 && !(mode != nullptr && mode[0] == 'l')) {  // bulk-copy engine path (rows are whole 16-byte multiples)
+  if (vec && tma_smem <= 56 * 1024 && count >= 4096) {  // bulk-copy engine path (rows are whole 16-byte multiples)
     static bool configured = false;
     if (!configured) {
       B2_CUDA(cudaFuncSetAttribute(gather_minibatch_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 56 * 1024));

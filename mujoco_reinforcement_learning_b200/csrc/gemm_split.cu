@@ -17,12 +17,8 @@
 // weight gradient (MN-major B operand).  Activations get a column of ones behind their last column (term a only): as the
 // weight gradient's B operand that column makes the bias gradient fall out of the same MMAs (TcProblem.bias_col).
 //
-// Environment switches (read once per process; all for measurements, none needed in use):
-//   B200PPO_FP32_TC=0              keep every fp32 GEMM on the FFMA kernels       B200PPO_FP32_TC_MIN_MACS   size threshold of the route
-//   B200PPO_SPLIT_TERMS=2|3        operand mode for every context (default: per context, b200ppo_set_fp32_terms)
-//   B200PPO_SPLIT_PERSIST=0        one-tile CTAs (tc_gemm_kernel) instead of the persistent kernel; then B200PPO_SPLIT_OCC[_WGRAD]=1|2
-//   B200PPO_SPLIT_BN[_WGRAD]       N tile       B200PPO_SPLIT_FUSE=0  no terms from the producing epilogue
-//   B200PPO_SPLIT_AXIS=1           two-term mode: one scale per row / column of the dL/dz operands instead of per tensor
+// Environment switches (read once per process; none needed in use):
+//   B200PPO_FP32_TC=0              keep every fp32 GEMM on the FFMA kernels
 //   B200PPO_SPLIT_TRACE=<n>        phase timeline of the n-th launch on stderr
 #include "gemm_split.cuh"
 
@@ -73,7 +69,6 @@ struct SplitJob {
   float* amax;                   // two-term mode: this operand's largest magnitude (filled by absmax_kernel, or from the bound)
   const float* bound_dev;        // a caller-supplied upper bound of it (device value; nullptr: `bound`; both empty: measure)
   float bound;
-  int axis;                      // 0: one scale for the operand; 1: amax[row]; 2: amax[column]
   int64_t rows, ld, unit_begin;  // first 8-column unit of this job in the launch
   int cols, cp, ones, vec, terms;
 };
@@ -202,50 +197,6 @@ __global__ void __launch_bounds__(256) colsum_kernel(const __grid_constant__ Col
   }
 }
 
-// Per-row / per-column magnitudes for operands whose rows (columns) differ by many powers of two — the dL/dz blocks: one
-// scale for the whole tensor would push the small rows' residual terms into fp16's subnormals, and what the optimizer sees
-// of a weight gradient is its error relative to ITS row, not to the tensor.  Units of these launches: axis 1 — one warp per
-// row; axis 2 — one thread per (four columns, 64 rows).
-__global__ void __launch_bounds__(256) axis_max_kernel(const __grid_constant__ SplitJobs jobs) {
-  const int64_t u = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (u >= jobs.units) return;
-  int ji = 0;
-#pragma unroll 1
-  for (int i = 1; i < jobs.n; ++i)
-    if (u >= jobs.j[i].unit_begin) ji = i;
-  const SplitJob& J = jobs.j[ji];
-  const int64_t local = u - J.unit_begin;
-  if (J.axis == 1) {  // unit_begin is a multiple of 32: whole warps
-    const int64_t row = local >> 5;
-    const int lane = int(local & 31);
-    float m = 0.f;
-    const float* sp = J.src + row * J.ld;
-    for (int c = lane; c < J.cols; c += 32) m = fmaxf(m, fabsf(__ldg(sp + c)));
-    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if (lane == 0) J.amax[row] = m;
-  } else {
-    const int groups = (J.cols + 3) >> 2;
-    const int64_t chunk = local / groups;
-    const int c0 = int(local - chunk * groups) * 4;
-    const int64_t r0 = chunk * 64, r1 = min(r0 + 64, J.rows);
-    float m[4] = {0.f, 0.f, 0.f, 0.f};
-    for (int64_t r = r0; r < r1; ++r) {
-      const float* sp = J.src + r * J.ld + c0;
-      if (J.vec && c0 + 4 <= J.cols) {
-        const float4 t = __ldg(reinterpret_cast<const float4*>(sp));
-        m[0] = fmaxf(m[0], fabsf(t.x)); m[1] = fmaxf(m[1], fabsf(t.y)); m[2] = fmaxf(m[2], fabsf(t.z)); m[3] = fmaxf(m[3], fabsf(t.w));
-      } else {
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-          if (c0 + j < J.cols) m[j] = fmaxf(m[j], fabsf(__ldg(sp + j)));
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-      if (c0 + j < J.cols && m[j] > 0.f) atomicMax(reinterpret_cast<unsigned*>(J.amax + c0 + j), __float_as_uint(m[j]));
-  }
-}
-
 __global__ void __launch_bounds__(256) split3_kernel(const __grid_constant__ SplitJobs jobs) {
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
@@ -264,26 +215,21 @@ __global__ void __launch_bounds__(256) split3_kernel(const __grid_constant__ Spl
   split_load8(J, row, c0, x, 1.f);
   if (J.terms == 2) {  // two fp16 terms of x * 2^e
     float am;
-    if (J.axis == 1) {
-      am = __ldg(J.amax + row);
-    } else if (J.bound_dev != nullptr || J.bound > 0.f) {  // no measuring pass ran: publish the bound for the GEMM's epilogue
+    if (J.bound_dev != nullptr || J.bound > 0.f) {  // no measuring pass ran: publish the bound for the GEMM's epilogue
       am = J.bound_dev != nullptr ? __ldg(J.bound_dev) : J.bound;
       if (J.ones) am = fmaxf(am, 1.f);
       if (u == J.unit_begin) *J.amax = am;
     } else {
       am = __ldg(J.amax);
     }
-    float scv[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j)
-      scv[j] = exp2f(float(split_exponent(J.axis == 2 ? ((c0 + j < J.cols) ? __ldg(J.amax + c0 + j) : 0.f) : am)));
+    const float sc = exp2f(float(split_exponent(am)));
     uint32_t o[2][4];
 #pragma unroll
     for (int j = 0; j < 8; j += 2) {
       __half t[2][2];
 #pragma unroll
       for (int k = 0; k < 2; ++k) {
-        float r = x[j + k] * scv[j + k];  // exact: a power of two, no overflow by the choice of e
+        float r = x[j + k] * sc;  // exact: a power of two, no overflow by the choice of e
 #pragma unroll
         for (int p = 0; p < 2; ++p) {
           t[p][k] = __float2half_rn(r);
@@ -321,11 +267,10 @@ __global__ void __launch_bounds__(256) split3_kernel(const __grid_constant__ Spl
 
 // Finds the split of (src, rows, cols, ld) in the arena or queues the job that makes it.
 static int get_split(SplitArena& arena, SplitJobs& jobs, const float* src, int64_t rows, int cols, int64_t ld, int ones, int terms,
-                     int axis, float bound, const float* bound_dev, const __nv_bfloat16** out, int* cp_out, const float** amax_out) {
-  if (terms != 2) axis = 0;
+                     float bound, const float* bound_dev, const __nv_bfloat16** out, int* cp_out, const float** amax_out) {
   for (int i = 0; i < arena.n; ++i) {
     const SplitArena::Entry& e = arena.e[i];
-    if (e.src == src && e.rows == rows && e.cols == cols && e.ld == ld && e.ones >= ones && e.terms == terms && e.axis == axis) {
+    if (e.src == src && e.rows == rows && e.cols == cols && e.ld == ld && e.ones >= ones && e.terms == terms) {
       *out = e.dst;
       *cp_out = e.cp;
       *amax_out = e.amax;
@@ -333,9 +278,7 @@ static int get_split(SplitArena& arena, SplitJobs& jobs, const float* src, int64
     }
   }
   const int cp = pad64(cols + 1);
-  // per-row / per-column magnitudes live behind the terms, as floats
-  const int64_t vec_floats = axis == 1 ? rows : (axis == 2 ? cols : 0);
-  const int64_t elems = split_arena_elems(rows, cols) + (2 * vec_floats + 511) / 512 * 512;
+  const int64_t elems = split_arena_elems(rows, cols);
   if (arena.n >= SplitArena::kMaxEntries || arena.used + elems > arena.cap || jobs.n >= kMaxSplitJobs) {
     set_error("three-term operand arena exhausted (%d entries, %lld of %lld elements used, %lld more asked)", arena.n,
               (long long)arena.used, (long long)arena.cap, (long long)elems);
@@ -343,12 +286,12 @@ static int get_split(SplitArena& arena, SplitJobs& jobs, const float* src, int64
   }
   __nv_bfloat16* dst = arena.base + arena.used;
   arena.used += elems;
-  float* am = axis == 0 ? arena.amax + arena.n : reinterpret_cast<float*>(dst + split_arena_elems(rows, cols));
+  float* am = arena.amax + arena.n;
   *amax_out = am;
-  arena.e[arena.n++] = SplitArena::Entry{src, rows, ld, cols, ones, cp, terms, axis, dst, am};
+  arena.e[arena.n++] = SplitArena::Entry{src, rows, ld, cols, ones, cp, terms, dst, am};
   SplitJob& J = jobs.j[jobs.n++];
   J.src = src; J.dst = dst; J.rows = rows; J.ld = ld; J.cols = cols; J.cp = cp; J.ones = ones;
-  J.terms = terms; J.amax = am; J.axis = axis;
+  J.terms = terms; J.amax = am;
   J.bound = bound; J.bound_dev = bound_dev;
   J.vec = (aligned16(src) && ld % 4 == 0) ? 1 : 0;
   J.unit_begin = jobs.units;
@@ -363,10 +306,6 @@ bool gemm_split_applicable(const GemmGroup& g) {
     const char* e = getenv("B200PPO_FP32_TC");
     return !(e != nullptr && e[0] == '0');
   }();
-  static const double min_macs = []() {
-    const char* e = getenv("B200PPO_FP32_TC_MIN_MACS");
-    return e != nullptr ? atof(e) : double(1ll << 27);
-  }();
   if (!on || g.count == 0 || g.count > kMaxTcProblems) return false;
   double macs = 0;
   for (int i = 0; i < g.count; ++i) {
@@ -379,17 +318,13 @@ bool gemm_split_applicable(const GemmGroup& g) {
     if (p.bias_grad != nullptr && !((a_mn && !a_k) && (b_mn && !b_k))) return false;  // bias gradients only off the wgrad layout
     macs += double(p.M) * p.N * p.K;
   }
-  return macs >= min_macs;
+  return macs >= double(1ll << 27);
 }
 
 int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t st) {
   if (g.total_tiles == 0 || g.count == 0) return B200PPO_OK;
   B2_TRY(tc_init());
-  static const int env_terms = []() {
-    const char* e = getenv("B200PPO_SPLIT_TERMS");
-    return e != nullptr ? atoi(e) : 0;
-  }();
-  const int terms = (env_terms == 2 || env_terms == 3) ? env_terms : (arena.terms == 2 ? 2 : 3);
+  const int terms = arena.terms == 2 ? 2 : 3;
   SplitJobs jobs{};
   ColsumJobs colsums{};
   TcGroup tg{};
@@ -401,13 +336,8 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
     maxN = std::max(maxN, g.p[i].N + ((g.p[i].bias_grad != nullptr && terms == 3) ? 1 : 0));
     any_wgrad |= g.p[i].bias_grad != nullptr;
   }
-  int BN = maxN <= 128 ? 128 : ((any_wgrad && terms == 3) ? 192 : 256);
-  if (const char* e = getenv(any_wgrad ? "B200PPO_SPLIT_BN_WGRAD" : "B200PPO_SPLIT_BN")) BN = atoi(e);
-  static const bool persist = []() {
-    const char* e = getenv("B200PPO_SPLIT_PERSIST");
-    return !(e != nullptr && e[0] == '0');
-  }();
-  const bool use_persist = persist && BN >= 192;
+  const int BN = maxN <= 128 ? 128 : ((any_wgrad && terms == 3) ? 192 : 256);
+  const bool use_persist = BN >= 192;  // one CTA per SM walks the tiles; the 128-wide tiles run one per CTA
   for (int i = 0; i < g.count; ++i) {
     const GemmProblem& p = g.p[i];
     const bool a_mn = !(p.a_sk == 1 && p.a_sm >= p.K), b_mn = !(p.b_sk == 1 && p.b_sn >= p.K);
@@ -415,20 +345,15 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
     const __nv_bfloat16 *As = nullptr, *Bs = nullptr;
     const float *a_amax = nullptr, *b_amax = nullptr;
     int a_cp = 0, b_cp = 0;
-    // the arrays as stored: K-major [M or N][K], MN-major [K][M or N]
-    // A operands of the backward GEMMs are dL/dz blocks: one scale per row of C (= per stored row for the dgrad's K-major view,
-    // per stored column for the weight gradient's MN-major view); everything else one scale per tensor
-    static const bool per_axis = getenv("B200PPO_SPLIT_AXIS") != nullptr;  // experiment switch; measured: no effect on parity, slower
-    const int a_axis = (fwd || !per_axis) ? 0 : (a_mn ? 2 : 1);
-    B2_TRY(get_split(arena, jobs, p.A, a_mn ? p.K : p.M, a_mn ? p.M : p.K, a_mn ? p.a_sk : p.a_sm, (fwd && terms == 3) ? 1 : 0, terms, a_axis, p.a_bound,
+    // the arrays as stored: K-major [M or N][K], MN-major [K][M or N]; one scale per tensor
+    B2_TRY(get_split(arena, jobs, p.A, a_mn ? p.K : p.M, a_mn ? p.M : p.K, a_mn ? p.a_sk : p.a_sm, (fwd && terms == 3) ? 1 : 0, terms, p.a_bound,
                      p.a_bound_dev, &As, &a_cp, &a_amax));
-    B2_TRY(get_split(arena, jobs, p.B, b_mn ? p.K : p.N, b_mn ? p.N : p.K, b_mn ? p.b_sk : p.b_sn, (wgrad && terms == 3) ? 1 : 0, terms, 0, p.b_bound,
+    B2_TRY(get_split(arena, jobs, p.B, b_mn ? p.K : p.N, b_mn ? p.N : p.K, b_mn ? p.b_sk : p.b_sn, (wgrad && terms == 3) ? 1 : 0, terms, p.b_bound,
                      p.b_bound_dev, &Bs, &b_cp, &b_amax));
     TcProblem t{};
     t.M = p.M; t.N = p.N; t.K = p.K;
     t.parts = terms; t.a_part = a_cp; t.b_part = b_cp;
     t.amax_a = a_amax; t.amax_b = b_amax;
-    t.a_scale_rows = (terms == 2 && a_axis != 0) ? 1 : 0;
     t.out_f32 = p.C; t.ld_f32 = p.ldc; t.split_stride = p.c_split_stride;
     t.bias_col = -1;
     t.out_scale = p.out_scale;
@@ -462,12 +387,8 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
     // Three-term mode: a hidden activation (forward) or a dL/dz block (dgrad) is the next GEMMs' operand — the epilogue writes
     // its terms straight into the arena (the persistent kernel's epilogue hides behind the next tile's main loop), which
     // saves the split pass over it.  (Two-term mode cannot: the scale is only known once the whole tensor exists.)
-    static const bool fuse_env = []() {
-      const char* e = getenv("B200PPO_SPLIT_FUSE");
-      return !(e != nullptr && e[0] == '0');
-    }();
     const bool producer = p.epilogue == EPI_BIAS_TANH || p.epilogue == EPI_BIAS_RELU || p.epilogue == EPI_DTANH || p.epilogue == EPI_DRELU;
-    if (fuse_env && use_persist && terms == 3 && producer && p.N % 16 == 0 && arena.n < SplitArena::kMaxEntries) {
+    if (use_persist && terms == 3 && producer && p.N % 16 == 0 && arena.n < SplitArena::kMaxEntries) {
       const int ocp = pad64(p.N + 1);
       const int64_t oelems = split_arena_elems(p.M, p.N);
       const int ones = (p.epilogue == EPI_BIAS_TANH || p.epilogue == EPI_BIAS_RELU) ? 1 : 0;
@@ -476,7 +397,7 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
       if (!known && arena.used + oelems <= arena.cap) {
         __nv_bfloat16* odst = arena.base + arena.used;
         arena.used += oelems;
-        arena.e[arena.n++] = SplitArena::Entry{p.C, int64_t(p.M), int64_t(p.ldc), p.N, ones, ocp, 3, 0, odst, arena.amax};
+        arena.e[arena.n++] = SplitArena::Entry{p.C, int64_t(p.M), int64_t(p.ldc), p.N, ones, ocp, 3, odst, arena.amax};
         t.out_split = odst; t.split_cp = ocp; t.split_ones = ones;
       }
     }
@@ -490,18 +411,9 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
         B2_CUDA(cudaMemsetAsync(arena.amax, 0, SplitArena::kMaxEntries * sizeof(float), st));
         arena.amax_zeroed = true;
       }
-      SplitJobs measure{}, axes{};  // the operands nobody gave a bound for; the ones scaled per row / per column
+      SplitJobs measure{};  // the operands nobody gave a bound for
       for (int i = 0; i < jobs.n; ++i) {
         const SplitJob& J = jobs.j[i];
-        if (J.axis != 0) {
-          SplitJob& Aj = axes.j[axes.n++];
-          Aj = J;
-          Aj.unit_begin = axes.units;
-          axes.units += J.axis == 1 ? J.rows * 32 : ((J.rows + 63) / 64) * ((J.cols + 3) / 4);
-          axes.units = (axes.units + 31) / 32 * 32;  // the next job starts on a warp
-          if (J.axis == 2) B2_CUDA(cudaMemsetAsync(J.amax, 0, size_t(J.cols) * sizeof(float), st));
-          continue;
-        }
         if (J.bound_dev != nullptr || J.bound > 0.f) continue;
         SplitJob& Mj = measure.j[measure.n++];
         Mj = J;
@@ -510,10 +422,6 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
       }
       if (measure.n > 0) {
         absmax_kernel<<<unsigned((measure.units + 255) / 256), 256, 0, st>>>(measure);
-        B2_LAUNCH_CHECK();
-      }
-      if (axes.n > 0) {
-        axis_max_kernel<<<unsigned((axes.units + 255) / 256), 256, 0, st>>>(axes);
         B2_LAUNCH_CHECK();
       }
     }
@@ -555,8 +463,7 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
     }
   } dump{trace, st, tg.total_tiles};
   // forward / dgrad: two CTAs per SM (two-stage rings); weight gradients: one CTA with the deep ring — measured, profiles/README.md
-  bool two = !any_wgrad;
-  if (const char* e = getenv(any_wgrad ? "B200PPO_SPLIT_OCC_WGRAD" : "B200PPO_SPLIT_OCC")) two = atoi(e) == 2;
+  const bool two = !any_wgrad;
   if (colsums.n > 0) {
     colsum_kernel<<<unsigned(colsums.blocks), 256, 0, st>>>(colsums);
     B2_LAUNCH_CHECK();

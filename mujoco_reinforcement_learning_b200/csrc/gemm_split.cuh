@@ -12,9 +12,9 @@ struct SplitArena {
   struct Entry {
     const float* src;
     int64_t rows, ld;
-    int cols, ones, cp, terms, axis;
+    int cols, ones, cp, terms;
     __nv_bfloat16* dst;
-    float* amax;  // scale source: one float (axis 0), one per row (1) or one per column (2)
+    float* amax;  // two-term mode: the largest magnitude of src, the source of its scale
   };
   static constexpr int kMaxEntries = 96;  // 2 nets x B200PPO_MAX_LAYERS x (activation, two dL/dz views, weights) and room to spare
   __nv_bfloat16* base = nullptr;

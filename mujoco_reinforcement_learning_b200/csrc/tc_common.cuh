@@ -136,7 +136,7 @@ __device__ __forceinline__ void tc_epilogue(const TcProblem& P, int split, uint3
     const bool aux_vec = (ld_aux % 8 == 0);
     // two-term fp16 mode: the operands were scaled by 2^eA and 2^eB
     const bool rescale = P.parts == 2;
-    const float acc_scale = rescale ? split_unscale(P.a_scale_rows ? (row_ok ? __ldg(P.amax_a + m) : 0.f) : __ldg(P.amax_a), __ldg(P.amax_b)) : 1.f;
+    const float acc_scale = rescale ? split_unscale(__ldg(P.amax_a), __ldg(P.amax_b)) : 1.f;
 
     uint4 pre[2];  // prefetched 32 bytes of the dgrad's activation row for the NEXT step
     float4 pref[CW / 4];  // the same for an fp32 activation operand (64 bytes)
@@ -397,7 +397,7 @@ template <int BN, bool TMA_OUT = false>
 __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split, uint32_t tmem_acc, bool has_k, int m0, int n0,
                                                    int warp, int lane, uint64_t* tmem_full_bar, uint32_t full_parity,
                                                    uint8_t* stage, const float* bias_s, int aux_groups_in_flight,
-                                                   const CUtensorMap* tm_out = nullptr, long long* tr = nullptr) {
+                                                   const CUtensorMap* tm_out = nullptr) {
   static_assert(BN == 64 || BN == 128, "staged epilogue: BN <= 128");
   constexpr int WCOLS = BN / 2, STEPS = WCOLS / 16, UPR = WCOLS / 8, RSTEP = 32 / UPR;
   (void)split;
@@ -417,7 +417,6 @@ __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   }
   __syncwarp();
-  if (tr != nullptr) tr[0] = clock64();  // accumulator ready
   const float* bs = bias_s + col0;
   // (loading the whole 64-column slab with one tcgen05.ld.x64 and a single wait was measured: no gain, +70 registers)
 #pragma unroll
@@ -429,7 +428,6 @@ __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split
 #pragma unroll
       for (int j = 0; j < 16; ++j) v[j] = 0u;
     }
-    if (tr != nullptr && s < 4) tr[1 + s] = clock64();  // TMEM load of step s returned
     uint32_t o[8];
     if (epi == TC_EPI_FWD) {
       float z[16];
@@ -462,7 +460,6 @@ __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split
     asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(my_row + uint32_t(((2 * s) ^ sw) << 4)), "r"(o[0]), "r"(o[1]), "r"(o[2]), "r"(o[3]) : "memory");
     asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(my_row + uint32_t(((2 * s + 1) ^ sw) << 4)), "r"(o[4]), "r"(o[5]), "r"(o[6]), "r"(o[7]) : "memory");
   }
-  if (tr != nullptr) tr[5] = clock64();  // math + staging writes done
   if constexpr (TMA_OUT) {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy st.shared -> visible to the copy engine
     __syncwarp();
@@ -636,7 +633,7 @@ template <int BN>
 __device__ __forceinline__ void tc_epilogue_ppo(const TcProblem& P, uint32_t tmem_acc, int m0, int warp, int lane,
                                                 uint64_t* tmem_full_bar, uint32_t full_parity, uint8_t* stage,
                                                 const float* bias_s, const float* consts_s, int groups_in_flight, PpoAcc& acc,
-                                                bool worker, long long* tr = nullptr) {
+                                                bool worker) {
   // worker: this warp processes the tile's rows of its TMEM lane quarter (the <= 32 output columns all sit in one
   // thread).  Two warps share a lane quarter: the one-tile kernel lets the first work; the persistent kernel
   // alternates tiles between the two warp groups.
@@ -645,7 +642,6 @@ __device__ __forceinline__ void tc_epilogue_ppo(const TcProblem& P, uint32_t tme
   const bool row_ok = m < P.M;
   if (groups_in_flight > 0) asm volatile("cp.async.wait_group 1;" ::: "memory");
   else asm volatile("cp.async.wait_group 0;" ::: "memory");
-  if (tr != nullptr) tr[0] = clock64();  // action slab landed
   // per-row scalars requested before the accumulator is awaited
   float old_lp = 0.f, adv = 0.f, tgt = 0.f;
   if (worker && row_ok) {
@@ -655,7 +651,6 @@ __device__ __forceinline__ void tc_epilogue_ppo(const TcProblem& P, uint32_t tme
   mbar_wait(tmem_full_bar, full_parity);
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   __syncwarp();
-  if (tr != nullptr) tr[1] = clock64();  // accumulator ready
   if (!worker) return;
   if (P.epilogue == TC_EPI_PPO_CRITIC) {
     uint32_t v[16];
@@ -691,7 +686,6 @@ __device__ __forceinline__ void tc_epilogue_ppo(const TcProblem& P, uint32_t tme
   else if (nch == 3) tc_ppo_actor_row<24>(P, tmem_acc, q, row_ok, old_lp, adv, act_s, dz_s, bias_s, consts_s, acc);
   else tc_ppo_actor_row<32>(P, tmem_acc, q, row_ok, old_lp, adv, act_s, dz_s, bias_s, consts_s, acc);
   __syncwarp();
-  if (tr != nullptr) tr[2] = clock64();  // row math done
   // coalesced store of the 32 x pitch bf16 seed slab (rows are adjacent in global memory)
   const int rows = min(32, P.M - mq);
   if (rows > 0) {

@@ -16,7 +16,6 @@
 // Operands may be K-major or MN-major (UMMA descriptor major bits), so forward (X W^T), dgrad (dZ W via a
 // transposed bf16 weight copy) and wgrad (dZ^T X, both operands MN-major) share the kernel with no transposes
 // of activations.
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -24,8 +23,6 @@
 #include "tc_common.cuh"
 
 namespace b200ppo {
-
-extern long long* g_ws_trace;
 
 // smem ring depth: K loops are 1-6 tiles for forward/dgrad, so for BN <= 128 two 32 KB stages + the 32 KB epilogue
 // staging area let two CTAs share an SM (one CTA's epilogue overlaps the other's TMA/MMA main loop); the wide tiles
@@ -363,12 +360,12 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
   p.M = M; p.N = N; p.K = K;
   p.epilogue = TC_EPI_STORE;
   p.out_f32 = part; p.ld_f32 = N; p.split_stride = stride; p.bias_col = -1;
-  // bn = -1: the persistent weights-stationary kernel; bn = -2: its forward (tanh, bf16) epilogue plus a clock64 timeline;
+  // bn = -1: the persistent weights-stationary kernel;
   // bn = -3: forward epilogue, C = float(tanh(A B^T) rounded to bf16) — the path the CTA-pair kernel takes for N > 128
   // bn = -4: dgrad epilogue, C on entry holds the activation operand h; C = float(bf16(A B^T * (1 - bf16(h)^2)))
+  B2_CHECK_ARG(bn >= 0 || bn == -1 || bn == -3 || bn == -4, "b200ppo_debug_tc_gemm: bn must be >= 0, -1, -3 or -4");
   const bool ws = bn < 0;
   const bool fwd_check = bn == -3 || bn == -4;
-  long long* trace = nullptr;
   if (bn == -4) {
     p.epilogue = TC_EPI_DGRAD; p.act = B200PPO_ACT_TANH;
     p.out_f32 = nullptr;
@@ -380,29 +377,14 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
     B2_LAUNCH_CHECK();
     p.ld_bf16 = int(ld); p.aux = auxb; p.ld_aux = int(ld);
   }
-  if (bn == -2 || bn == -3) {
+  if (bn == -3) {
     p.epilogue = TC_EPI_FWD; p.act = B200PPO_ACT_TANH;  // the production forward epilogue, bf16 output
-    if (getenv("B200PPO_DEBUG_RELU") != nullptr) p.act = B200PPO_ACT_RELU;  // profiling: the epilogue without MUFU work
-    if (getenv("B200PPO_DEBUG_DGRAD") != nullptr) {  // profiling: the dgrad epilogue (activation operand = the output buffer's twin)
-      p.epilogue = TC_EPI_DGRAD;
-      __nv_bfloat16* auxb = nullptr;
-      B2_CUDA(cudaMalloc(&auxb, size_t(M) * ((N + 7) / 8 * 8) * 2));
-      B2_CUDA(cudaMemset(auxb, 0x3c, size_t(M) * ((N + 7) / 8 * 8) * 2));
-      p.aux = auxb; p.ld_aux = (N + 7) / 8 * 8;
-    }
     p.out_f32 = nullptr;
     B2_CUDA(cudaMalloc(&p.out_bf16, size_t(M) * ((N + 7) / 8 * 8) * 2));
     p.ld_bf16 = (N + 7) / 8 * 8;
-    if (bn == -2) {
-      B2_CUDA(cudaMalloc(&trace, 64 * 16 * sizeof(long long)));
-      B2_CUDA(cudaMemset(trace, 0, 64 * 16 * sizeof(long long)));
-      g_ws_trace = trace;
-    }
   }
   if (ws) bn = tc_ws_bn(N, K);
   int rc = tc_group_add(g, p, TcOperand{Ab, a_pitch, a_mn_major}, TcOperand{Bb, b_pitch, b_mn_major}, bn, split_k);
-  if (rc == B200PPO_OK && ws && getenv("B200PPO_DEBUG_TWICE") != nullptr)  // profiling: two problems per launch, like actor + critic
-    rc = tc_group_add(g, p, TcOperand{Ab, a_pitch, a_mn_major}, TcOperand{Bb, b_pitch, b_mn_major}, bn, split_k);
   if (rc == B200PPO_OK) rc = ws ? launch_tc_ws(g, st) : launch_tc_group(g, bn, st);
   if (rc == B200PPO_OK && fwd_check) {
     bf16_rows_to_f32_kernel<<<unsigned((mn + 255) / 256), 256, 0, st>>>(p.out_bf16, M, N, p.ld_bf16, C);
@@ -412,24 +394,6 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
     count_launch();
   }
   cudaStreamSynchronize(st);
-  if (trace != nullptr) {
-    long long h[64 * 16];
-    cudaMemcpy(h, trace, sizeof(h), cudaMemcpyDeviceToHost);
-    const long long t0 = h[0];
-    fprintf(stderr, "WS timeline of CTA 0 (cycles since first issue): tile | prod_first prod_last | mma_acc_free mma_kb0 mma_kbN | epi_start epi_end(w2) epi_end(slowest)\n");
-    for (int t = 0; t < 63 && h[t * 16] != 0; ++t) {
-      fprintf(stderr, "  %2d | %7lld %7lld | %7lld %7lld %7lld | %7lld %7lld %7lld", t, h[t * 16] - t0, h[t * 16 + 1] - t0, h[t * 16 + 2] - t0,
-              h[t * 16 + 3] - t0, h[t * 16 + 4] - t0, h[t * 16 + 5] - t0, h[t * 16 + 6] - t0, h[t * 16 + 7] - t0);
-      // warp 2's epilogue phases: accumulator ready, the four TMEM loads returned, staging written
-      fprintf(stderr, " | %7lld %7lld %7lld %7lld %7lld %7lld\n", h[t * 16 + 8] - t0, h[t * 16 + 9] - t0, h[t * 16 + 10] - t0, h[t * 16 + 11] - t0,
-              h[t * 16 + 12] - t0, h[t * 16 + 13] - t0);
-    }
-    if (h[63 * 16] != 0)
-      fprintf(stderr, "  kernel entry %lld | set-up done %lld | W resident %lld | kernel end %lld\n", h[63 * 16] - t0, h[63 * 16 + 1] - t0,
-              h[63 * 16 + 2] - t0, h[63 * 16 + 3] - t0);
-    g_ws_trace = nullptr;
-    cudaFree(trace);
-  }
   if (p.out_bf16 != nullptr) cudaFree(p.out_bf16);
   if (p.aux != nullptr) cudaFree(const_cast<__nv_bfloat16*>(p.aux));
   cudaFree(Ab); cudaFree(Bb); cudaFree(part);

@@ -69,7 +69,6 @@ struct TcProblem {
   // the zero padding (and the ones-column, split_ones) of gemm_split.cu's layout — the next GEMM's operand without a split pass
   __nv_bfloat16* out_split;
   int split_cp, split_ones;
-  int a_scale_rows;  // amax_a is a vector with one entry per row of C (the A operand was scaled per row / per column)
   const float* aux_f32;  // TC_EPI_DGRAD: activation operand in fp32 (instead of `aux`)
   int precise;           // TC_EPI_FWD: tanhf instead of the MUFU approximation
   TcPpo ppo;

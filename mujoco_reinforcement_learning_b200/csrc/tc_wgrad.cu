@@ -253,41 +253,11 @@ int launch_tc_wgrad2(const TcGroup& g, int max_split, cudaStream_t st, int* spli
   if (w.n_tiles == 0) return B200PPO_OK;
   const int total_kt = int((K + TC_BK - 1) / TC_BK);
   const int pairs = num_sms() / 2;
-  // bytes a pair streams per k-tile for every block (rows / columns past the matrix are zero-filled without traffic)
-  double weight[kWg2MaxTiles], wsum = 0.0;
-  for (int t = 0; t < w.n_tiles; ++t) {
-    const Wg2Tile& T = w.tile[t];
-    const TcProblem& p = w.p[T.prob];
-    const int rows = std::min(2 * TC_BM, p.M - T.m0), cols = std::min(T.nw, p.N - T.n0);
-    weight[t] = double(rows + cols) * TC_BK * 2 + 2048.0;  // + a little for the per-k-tile fixed cost
-    wsum += weight[t];
-  }
-  // Measured (profiles/README.md, round 2): splits in proportion to the bytes a block streams are SLOWER than the same
-  // split for every block (8.28 vs 7.07 ms per 160 launches) — with a common split all blocks walk the batch in step, so
-  // the operands two blocks share (dZ1 of the two dW1 blocks, every k-tile of X / H) meet in L2.  Uniform is the default;
-  // B200PPO_WGRAD_UNIFORM=0 selects the weighted split.
-  static const char* uni_env = getenv("B200PPO_WGRAD_UNIFORM");
-  const bool uniform = !(uni_env != nullptr && uni_env[0] == '0');
-  const char* uni = uniform ? "1" : nullptr;
-  int used = 0, max_sp = 1;
-  for (int t = 0; t < w.n_tiles; ++t) {
-    int sp = (uni != nullptr && uni[0] == '1') ? pairs / w.n_tiles : int(pairs * weight[t] / wsum);
-    sp = std::max(1, std::min({sp, max_split, total_kt}));
-    w.tile[t].splits = sp;
-    used += sp;
-  }
-  // hand the pairs the rounding left over to the blocks with the most bytes per pair
-  while (used < pairs && !(uni != nullptr && uni[0] == '1')) {
-    int best = -1;
-    double worst = 0.0;
-    for (int t = 0; t < w.n_tiles; ++t) {
-      const double per_pair = weight[t] / w.tile[t].splits;
-      if (w.tile[t].splits < std::min(max_split, total_kt) && per_pair > worst) { worst = per_pair; best = t; }
-    }
-    if (best < 0) break;
-    ++w.tile[best].splits;
-    ++used;
-  }
+  // The same split for every block: all blocks then walk the batch in step, so the operands two blocks share (dZ1 of the
+  // two dW1 blocks, every k-tile of X / H) meet in L2.  Measured (profiles/README.md, round 2): splits in proportion to
+  // the bytes a block streams were slower (8.28 vs 7.07 ms per 160 launches).
+  int max_sp = 1;
+  for (int t = 0; t < w.n_tiles; ++t) w.tile[t].splits = std::max(1, std::min({pairs / w.n_tiles, max_split, total_kt}));
   int begin = 0;
   for (int t = 0; t < w.n_tiles; ++t) {
     Wg2Tile& T = w.tile[t];

@@ -10,7 +10,6 @@
 //   warp 1      MMA issuer (one lane): tcgen05.mma M=128, N=BN, K=16, commit -> frees the A stage / publishes the tile
 //   warps 2-9   epilogue (shared with tc_gemm.cu): tcgen05.ld, bias + MUFU tanh | act' multiply, bf16/fp32 stores
 #include <algorithm>
-#include <cstdlib>
 
 #include "tc_common.cuh"
 
@@ -25,20 +24,11 @@ struct WsGroup {
   int n_slots;
   int slot_prob[kWsMaxSlots], slot_n0[kWsMaxSlots];
   int cta_begin[kWsMaxSlots + 1];  // CTAs [cta_begin[i], cta_begin[i+1]) serve slot i
-  long long* trace;                // debug: clock64 timeline of CTA 0, [tile][16] (nullptr in production)
   CUtensorMap tm_out[2];           // per problem: bf16 output as 64-column x 32-row swizzled boxes (bulk-store epilogue)
   int tma_out[2];                  // the problem's epilogue leaves through tm_out
   int stage_tiles;                 // 4 KB staging tiles per epilogue warp (2, or 3 when a dgrad's weights leave room)
   int w_early;                     // the stationary weights were written >= 2 kernels back: load them before the PDL wait
 };
-
-long long* g_ws_trace = nullptr;  // set by the debug entry point only
-
-#define WS_TRACE(tile_idx, slot_idx)                                                        \
-  do {                                                                                      \
-    if (grp.trace != nullptr && blockIdx.x == 0 && (tile_idx) < 63) grp.trace[(tile_idx) * 16 + (slot_idx)] = clock64(); \
-  } while (0)
-
 
 template <int BN>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_constant__ WsGroup grp, int a_stages) {
@@ -112,16 +102,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
     if (lane == 0) {  // ===== TMA producer =====
       if (!grp.w_early) load_w();
       int it = 0;
-      int tt = 0;
-      for (int tile = cta_local; tile < tiles_m; tile += ctas, ++tt) {
+      for (int tile = cta_local; tile < tiles_m; tile += ctas) {
         for (int kb = 0; kb < KB; ++kb, ++it) {
           const int s = it % a_stages;
           const uint32_t ph = (it / a_stages) & 1;
           mbar_wait(&a_empty[s], ph ^ 1);
-          if (kb == 0) WS_TRACE(tt, 0);
           mbar_expect_tx(&a_full[s], TC_A_BYTES);
           tma_load_2d(sA + size_t(s) * TC_A_BYTES, &P.tmA, &a_full[s], kb * TC_BK, tile * TC_BM);
-          if (kb == KB - 1) WS_TRACE(tt, 1);
         }
       }
     }
@@ -136,14 +123,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
         const int buf = t & 1;
         mbar_wait(&acc_empty[buf], ((t >> 1) & 1) ^ 1);  // epilogue has drained this accumulator
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        WS_TRACE(t, 2);
         for (int kb = 0; kb < KB; ++kb, ++it) {
           const int s = it % a_stages;
           const uint32_t ph = (it / a_stages) & 1;
           mbar_wait(&a_full[s], ph);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          if (kb == 0) WS_TRACE(t, 3);
-          if (kb == KB - 1) WS_TRACE(t, 4);
           const uint32_t a_addr = smem_u32(sA + size_t(s) * TC_A_BYTES), b_addr = smem_u32(sW + size_t(kb) * W_KB_BYTES);
 #pragma unroll
           for (int k = 0; k < TC_BK / 16; ++k)
@@ -172,12 +156,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
         for (; tile < tiles_m; tile += step, ++u) {
           const int next = tile + step;
           tc_ppo_issue(P, next * TC_BM, warp, lane, st[(u & 1) ^ 1], next < tiles_m);
-          if ((warp & 3) == 2 && lane == 0) WS_TRACE(2 * u + grp_id, 5);
           tc_epilogue_ppo<BN>(P, tmem_base + uint32_t(grp_id * BN), tile * TC_BM, warp, lane, &acc_full[grp_id], uint32_t(u & 1),
-                              st[u & 1], bias_s, consts_s, 1, acc, true,
-                              (grp.trace != nullptr && blockIdx.x == 0 && (warp & 3) == 2 && lane == 0 && 2 * u + grp_id < 63)
-                                  ? grp.trace + (2 * u + grp_id) * 16 + 8 : nullptr);
-          if ((warp & 3) == 2 && lane == 0) WS_TRACE(2 * u + grp_id, 6);
+                              st[u & 1], bias_s, consts_s, 1, acc, true);
           asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
           __syncwarp();
           if (lane == 0) mbar_arrive(&acc_empty[grp_id]);
@@ -199,7 +179,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
           const int nxt_i = cur_i + 1 == ntiles ? 0 : cur_i + 1;
           uint8_t* cur = st_base + cur_i * TC_STAGE_BYTES;
           uint8_t* nxt = st_base + nxt_i * TC_STAGE_BYTES;
-          if (warp == 2 && lane == 0) WS_TRACE(t, 5);
           if (tma_out) {
             // tile `cur` was last read by the bulk store of row tile t - ntiles, `nxt` by that of t + 1 - ntiles
             if (lane == 0) {
@@ -211,15 +190,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
           tc_issue_aux<BN>(P, next * TC_BM, n0, warp, lane, nxt, next < tiles_m);
           if (tma_out)
             tc_epilogue_staged<BN, BN == 128>(P, 0, tmem_base + uint32_t(buf * BN), true, tile * TC_BM, n0, warp, lane, &acc_full[buf],
-                                              uint32_t((t >> 1) & 1), cur, bias_s, 1, tm_out,
-                                              (grp.trace != nullptr && blockIdx.x == 0 && warp == 2 && lane == 0 && t < 64) ? grp.trace + t * 16 + 8 : nullptr);
+                                              uint32_t((t >> 1) & 1), cur, bias_s, 1, tm_out);
           else
             tc_epilogue_staged<BN>(P, 0, tmem_base + uint32_t(buf * BN), true, tile * TC_BM, n0, warp, lane, &acc_full[buf],
                                    uint32_t((t >> 1) & 1), cur, bias_s, 1);
           cur_i = nxt_i;
-          if (warp == 2 && lane == 0) WS_TRACE(t, 6);
-          if (lane == 0 && grp.trace != nullptr && blockIdx.x == 0 && t < 64)  // slowest epilogue warp of the tile
-            atomicMax(reinterpret_cast<unsigned long long*>(grp.trace) + t * 16 + 7, (unsigned long long)clock64());
         } else {
           tc_epilogue<BN>(P, 0, tmem_base + uint32_t(buf * BN), true, tile * TC_BM, n0, warp, lane, &acc_full[buf], uint32_t((t >> 1) & 1), bias_s);
         }
@@ -273,7 +248,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
-  if (grp.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0) grp.trace[63 * 16] = clock64();  // kernel entry
   int slot = 0;
 #pragma unroll 1
   for (int i = 1; i < grp.n_slots; ++i)
@@ -312,7 +286,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
   cluster_sync_all();  // both CTAs' barriers exist before any remote arrive / TMA completion targets them
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
-  if (grp.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0) grp.trace[63 * 16 + 1] = clock64();  // set-up done
   const bool w_early = grp.w_early != 0;
   if (!(warp == 0 && lane == 0 && w_early)) pdl_wait_then_release();  // the producer lane first requests W (below)
   if (warp >= 2) {  // epilogue warps stage the bias (named barrier 1)
@@ -345,8 +318,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
           const int s = it % a_stages;
           const uint32_t ph = (it / a_stages) & 1;
           mbar_wait(&a_empty[s], ph ^ 1);
-          if (kb == 0) WS_TRACE(tt, 0);
-          if (kb == KB - 1) WS_TRACE(tt, 1);
           if (tt == 0 && !w_early) load_w(kb);  // W k-block and the first tile's A k-block interleaved: the MMA needs them in this order
           if (rank == 0) mbar_expect_tx(&a_full[s], 2u * TC_A_BYTES);
           tma_load_2d_pair(sA + size_t(s) * TC_A_BYTES, &P.tmA, mapa_u32(smem_u32(&a_full[s]), 0), kb * TC_BK, m0);
@@ -363,18 +334,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
         const int buf = t & 1;
         mbar_wait(&acc_empty[buf], ((t >> 1) & 1) ^ 1);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        WS_TRACE(t, 2);
         for (int kb = 0; kb < KB; ++kb, ++it) {
           const int s = it % a_stages;
           const uint32_t ph = (it / a_stages) & 1;
-          if (t == 0) {
-            mbar_wait(&w_full[kb], 0);
-            if (kb == KB - 1 && grp.trace != nullptr && blockIdx.x == 0) grp.trace[63 * 16 + 2] = clock64();  // all of W resident
-          }
+          if (t == 0) mbar_wait(&w_full[kb], 0);
           mbar_wait(&a_full[s], ph);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          if (kb == 0) WS_TRACE(t, 3);
-          if (kb == KB - 1) WS_TRACE(t, 4);
           const uint32_t a_addr = smem_u32(sA + size_t(s) * TC_A_BYTES), b_addr = smem_u32(sW + size_t(kb) * W_KB_BYTES);
 #pragma unroll
           for (int k = 0; k < TC_BK / 16; ++k)
@@ -493,7 +458,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
       tile_i = tile_i + 1 == ntiles ? 0 : tile_i + 1;
       const uint32_t sbase = smem_u32(st), my_row = sbase + uint32_t(lane) * 128u;
       const uint32_t tcol = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(buf * BN + col0);
-      if (warp == 2 && lane == 0) WS_TRACE(t, 5);
       // the bulk store that last read this staging tile (ntiles row tiles ago) must have drained it
       if (lane == 0) {
         if (ntiles == 1) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
@@ -502,7 +466,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
       mbar_wait(&acc_full[buf], uint32_t((t >> 1) & 1));
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       __syncwarp();
-      if (warp == 2 && lane == 0) WS_TRACE(t, 8);
       uint32_t va[16], vb[16];
       tmem_ld16_nowait(tcol, va);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
@@ -531,16 +494,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
         }
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
       }
-      if (warp == 2 && lane == 0) WS_TRACE(t, 9);
-      if (lane == 0 && grp.trace != nullptr && blockIdx.x == 0 && t < 63)
-        atomicMax(reinterpret_cast<unsigned long long*>(grp.trace) + t * 16 + 7, (unsigned long long)clock64());
     }
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   cluster_sync_all();  // the peer may still be reading this CTA's operands / arriving on its barriers
-  if (grp.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0) grp.trace[63 * 16 + 3] = clock64();  // kernel end
   if (warp == 2) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
@@ -621,18 +580,15 @@ int launch_tc_ws(const TcGroup& g, cudaStream_t st, int* grid_out, bool w_early)
     maxN = std::max(maxN, g.p[i].N);
     maxK = std::max(maxK, g.p[i].K);
   }
-  static const char* store_mode = getenv("B200PPO_WS_STORE");  // profiling switch: "lsu" keeps the load/store epilogue
-  const bool bulk_store = !(store_mode != nullptr && store_mode[0] == 'l');
   int kind = 0;  // all problems staged forward -> 0; any dgrad -> 1; anything else -> 2
   for (int i = 0; i < g.count; ++i) {
     if (g.p[i].epilogue == TC_EPI_DGRAD) kind = std::max(kind, 1);
-    else if (!(g.p[i].epilogue == TC_EPI_FWD && g.p[i].staged && bulk_store)) kind = 2;
+    else if (!(g.p[i].epilogue == TC_EPI_FWD && g.p[i].staged)) kind = 2;
   }
   int bn, stages, stage_tiles;
   ws_plan(maxN, maxK, kind, &bn, &stages, &stage_tiles, tc_ws_bn(maxN, maxK));
   // CTA pairs with 256-wide MMAs for wide forward layers (every problem N > 128, operands built for 128-row boxes)
-  static const char* pair_mode = getenv("B200PPO_WS_PAIR");  // profiling switch: "0" keeps the single-CTA kernel
-  bool pair = (kind == 0 || kind == 1) && bn == 128 && !(pair_mode != nullptr && pair_mode[0] == '0');
+  bool pair = (kind == 0 || kind == 1) && bn == 128;
   for (int i = 0; i < g.count; ++i) {
     const TcProblem& q = g.p[i];
     pair = pair && q.N > 128 && q.tiles_m >= 2;
@@ -644,8 +600,7 @@ int launch_tc_ws(const TcGroup& g, cudaStream_t st, int* grid_out, bool w_early)
   int pair_stages = 0;
   // forward epilogue: 256-bit stores straight from registers when every row segment is a whole, aligned 32-byte sector
   // (measured 3% faster than staging + bulk store, and the staging tiles' shared memory goes to the A ring instead)
-  static const char* fwd_mode = getenv("B200PPO_WS_FWD");  // profiling switch: "tma" keeps the staged bulk-store epilogue
-  bool fwd_direct = kind == 0 && !(fwd_mode != nullptr && fwd_mode[0] == 't');
+  bool fwd_direct = kind == 0;
   for (int i = 0; i < g.count; ++i)
     fwd_direct = fwd_direct && g.p[i].N % 64 == 0 && g.p[i].ld_bf16 % 16 == 0 && (reinterpret_cast<uintptr_t>(g.p[i].out_bf16) & 31u) == 0;
   const int pair_tiles = (kind == 1 || fwd_direct) ? 0 : 1;  // staged forward: one tile per epilogue warp (a whole row tile to drain)
@@ -687,7 +642,6 @@ int launch_tc_ws(const TcGroup& g, cudaStream_t st, int* grid_out, bool w_early)
     }
     const int total_pairs = std::max(begin, pairs_total);
     w.cta_begin[w.n_slots] = 2 * total_pairs;
-    w.trace = g_ws_trace;
     const int smem = pair_kb * 128 * TC_BK * 2 + pair_stages * TC_A_BYTES + ws2_fixed_smem(pair_tiles);
     static int configured = 0;
     if (configured < smem) {
@@ -707,7 +661,7 @@ int launch_tc_ws(const TcGroup& g, cudaStream_t st, int* grid_out, bool w_early)
   for (int i = 0; i < g.count; ++i) {
     const TcProblem& q = g.p[i];
     w.tma_out[i] = 0;
-    if (bn == 128 && q.staged && bulk_store) {
+    if (bn == 128 && q.staged) {
       B2_TRY(tc_make_map(&w.tm_out[i], q.out_bf16, q.N, q.M, q.ld_bf16, 64, 32));
       w.tma_out[i] = 1;
     }
@@ -732,32 +686,9 @@ int launch_tc_ws(const TcGroup& g, cudaStream_t st, int* grid_out, bool w_early)
     begin += share;
   }
   w.cta_begin[w.n_slots] = std::max(begin, grid);
-  w.trace = g_ws_trace;
   const int kb_max = (maxK + TC_BK - 1) / TC_BK;
   const int total = w.cta_begin[w.n_slots];
   if (grid_out) *grid_out = total;
-  // profiling aid: B200PPO_WS_TRACE=ppo prints the clock64 timeline of CTA 0 of the 20th fused-loss output-layer launch
-  static const char* trace_mode = getenv("B200PPO_WS_TRACE");
-  if (trace_mode != nullptr && trace_mode[0] == 'p' && bn == 64 && g.p[0].epilogue >= TC_EPI_PPO_ACTOR) {
-    static int calls = 0;
-    if (++calls == 20) {
-      long long* tr = nullptr;
-      B2_CUDA(cudaMalloc(&tr, 64 * 16 * sizeof(long long)));
-      B2_CUDA(cudaMemset(tr, 0, 64 * 16 * sizeof(long long)));
-      w.trace = tr;
-      const int rc = launch_ws_bn<64>(w, stages, kb_max, total, st);
-      cudaStreamSynchronize(st);
-      long long h[64 * 16];
-      cudaMemcpy(h, tr, sizeof(h), cudaMemcpyDeviceToHost);
-      const long long t0 = h[0];
-      fprintf(stderr, "fused-loss output layer, CTA 0: tile | prod_first prod_last | mma_acc_free mma_kb0 mma_kbN | epi_start epi_end\n");
-      for (int t = 0; t < 16 && h[t * 16] != 0; ++t)
-        fprintf(stderr, "  %2d | %7lld %7lld | %7lld %7lld %7lld | %7lld %7lld | slab %7lld acc %7lld math %7lld\n", t, h[t * 16] - t0, h[t * 16 + 1] - t0, h[t * 16 + 2] - t0,
-                h[t * 16 + 3] - t0, h[t * 16 + 4] - t0, h[t * 16 + 5] - t0, h[t * 16 + 6] - t0, h[t * 16 + 8] - t0, h[t * 16 + 9] - t0, h[t * 16 + 10] - t0);
-      cudaFree(tr);
-      return rc;
-    }
-  }
   switch (bn) {
     case 64: return launch_ws_bn<64>(w, stages, kb_max, total, st);
     case 128: return launch_ws_bn<128>(w, stages, kb_max, total, st);
