@@ -78,8 +78,7 @@ __device__ __forceinline__ void add_partials(float4& g, const float* __restrict_
 struct CastTable {
   int64_t begin[2 * B200PPO_MAX_LAYERS], end[2 * B200PPO_MAX_LAYERS];  // element range of each matrix in the flat buffer
   __nv_bfloat16* dst[2 * B200PPO_MAX_LAYERS];
-  __nv_bfloat16* dst_t[2 * B200PPO_MAX_LAYERS];
-  int in[2 * B200PPO_MAX_LAYERS], pitch[2 * B200PPO_MAX_LAYERS], pitch_t[2 * B200PPO_MAX_LAYERS];
+  int in[2 * B200PPO_MAX_LAYERS], pitch[2 * B200PPO_MAX_LAYERS];
   int count;
 };
 
@@ -231,7 +230,7 @@ adam_cast_kernel(float* __restrict__ params, const float* __restrict__ grads, in
 #pragma unroll 1
     for (int c = 0; c < ct.count; ++c)
       if (e >= ct.begin[c] && e < ct.end[c]) k = c;
-    if (k >= 0 && ct.dst_t[k] == nullptr && (ct.in[k] & 3) == 0 && (ct.pitch[k] & 3) == 0 && e + 3 < ct.end[k]) {
+    if (k >= 0 && (ct.in[k] & 3) == 0 && (ct.pitch[k] & 3) == 0 && e + 3 < ct.end[k]) {
       // whole float4 inside one row (rows are multiples of 4 wide): one 32-bit division, one 8-byte store
       const uint32_t in = uint32_t(ct.in[k]), rel = uint32_t(e - ct.begin[k]);
       const uint32_t o = rel / in, c2 = rel - o * in;
@@ -248,9 +247,7 @@ adam_cast_kernel(float* __restrict__ params, const float* __restrict__ grads, in
       for (int j = 0; j < 4; ++j) {
         if (e + j >= ct.end[k]) break;
         const int o = int((rel + j) / in), c2 = int((rel + j) - int64_t(o) * in);
-        const __nv_bfloat16 b = __float2bfloat16_rn(pv[j]);
-        ct.dst[k][int64_t(o) * ct.pitch[k] + c2] = b;
-        if (ct.dst_t[k] != nullptr) ct.dst_t[k][int64_t(c2) * ct.pitch_t[k] + o] = b;
+        ct.dst[k][int64_t(o) * ct.pitch[k] + c2] = __float2bfloat16_rn(pv[j]);
       }
     }
   }
@@ -337,8 +334,8 @@ int launch_adam_cast(float* params, const float* grads, int n_partials, int64_t 
     ct.begin[k] = w.src - params;
     ct.end[k] = ct.begin[k] + int64_t(w.out) * w.in;
     B2_CHECK_ARG(ct.begin[k] >= 0 && ct.end[k] <= n, "weight cast source outside the parameter buffer");
-    ct.dst[k] = w.dst; ct.dst_t[k] = w.dst_t;
-    ct.in[k] = w.in; ct.pitch[k] = w.pitch; ct.pitch_t[k] = w.pitch_t;
+    ct.dst[k] = w.dst;
+    ct.in[k] = w.in; ct.pitch[k] = w.pitch;
   }
   B2_CHECK_ARG(peers == nullptr || peers->local_out == nullptr || int64_t(ew_grid(n / 4)) * 256 >= n / 4,
                "fused reduce + exchange: one element per thread");

@@ -175,7 +175,6 @@ struct b200ppo_ctx {
     __nv_bfloat16* H[2][B200PPO_MAX_LAYERS] = {};   // hidden activations [max_batch, pitchH], ones in column dims[l]
     __nv_bfloat16* dZ[2][B200PPO_MAX_LAYERS] = {};  // dL/dz of every layer [max_batch, pitchZ]
     __nv_bfloat16* W[2][B200PPO_MAX_LAYERS] = {};   // W_l   [dims[l], pitchW]
-    __nv_bfloat16* WT[2][B200PPO_MAX_LAYERS] = {};  // W_l^T [in_l, pitchZ] (l >= 1)
     int pitchH[2][B200PPO_MAX_LAYERS] = {}, pitchZ[2][B200PPO_MAX_LAYERS] = {}, pitchW[2][B200PPO_MAX_LAYERS] = {};
     __nv_bfloat16* X = nullptr;      // [max_batch, pitchX] staged observations (grads-only entry point)
     __nv_bfloat16* sh_obs = nullptr; // [sh_cap, pitchX] shuffled observations of an epoch
@@ -435,8 +434,8 @@ static int alloc_bf16_workspaces(b200ppo_ctx* c) {
       B2_TRY(dev_alloc(&bf.W[n][l], int64_t(N.d.dims[l]) * bf.pitchW[n][l], true));
       WeightCast& w = bf.casts.w[bf.casts.count++];
       w.src = nullptr;  // the parameter base is a per-call argument: filled in by cast_weights()
-      w.dst = bf.W[n][l]; w.dst_t = bf.WT[n][l];
-      w.out = N.d.dims[l]; w.in = N.in_dim(l); w.pitch = bf.pitchW[n][l]; w.pitch_t = bf.pitchZ[n][l];
+      w.dst = bf.W[n][l];
+      w.out = N.d.dims[l]; w.in = N.in_dim(l); w.pitch = bf.pitchW[n][l];
       bf.casts.max_elems = std::max(bf.casts.max_elems, w.out * w.in);
     }
   }
@@ -933,7 +932,7 @@ extern "C" B2_EXPORT void b200ppo_destroy(b200ppo_ctx* c) {
   dev_free(c->rollout_tmp);
   split_arena_free(c->arena);
   for (int n = 0; n < 2; ++n)
-    for (int l = 0; l < B200PPO_MAX_LAYERS; ++l) { dev_free(c->bf.H[n][l]); dev_free(c->bf.dZ[n][l]); dev_free(c->bf.W[n][l]); dev_free(c->bf.WT[n][l]); }
+    for (int l = 0; l < B200PPO_MAX_LAYERS; ++l) { dev_free(c->bf.H[n][l]); dev_free(c->bf.dZ[n][l]); dev_free(c->bf.W[n][l]); }
   dev_free(c->bf.X); dev_free(c->bf.sh_obs); dev_free(c->bf.obs_table); dev_free(c->replica);
   dev_free(c->sh_obs); dev_free(c->sh_act); dev_free(c->sh_logp); dev_free(c->sh_adv); dev_free(c->sh_tgt);
   for (auto& h : c->host) {

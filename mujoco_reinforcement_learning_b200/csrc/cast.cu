@@ -1,6 +1,6 @@
 // bf16 shadow copies of the fp32 master weights and bf16 staging of observations for the tcgen05 path.
 // The optimiser keeps fp32 master parameters (b200ppo_adam_step); after every step the hidden-layer weights are
-// re-emitted as bf16 in the two layouts the tensor-core GEMMs consume (W for forward, W^T for dgrad).
+// re-emitted as bf16 (W as is: K-major for the forward GEMMs, MN-major for the dgrad).
 #include <algorithm>
 
 #include "cast.cuh"
@@ -12,9 +12,7 @@ __global__ void __launch_bounds__(256) cast_weights_kernel(const __grid_constant
   const int total = w.out * w.in;
   for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < total; e += gridDim.x * blockDim.x) {
     const int o = e / w.in, i = e - o * w.in;
-    const __nv_bfloat16 v = __float2bfloat16_rn(__ldg(w.src + e));
-    w.dst[int64_t(o) * w.pitch + i] = v;
-    if (w.dst_t != nullptr) w.dst_t[int64_t(i) * w.pitch_t + o] = v;
+    w.dst[int64_t(o) * w.pitch + i] = __float2bfloat16_rn(__ldg(w.src + e));
   }
 }
 

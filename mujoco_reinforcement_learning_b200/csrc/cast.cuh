@@ -8,9 +8,8 @@ namespace b200ppo {
 
 struct WeightCast {
   const float* src;        // W [out, in] fp32 (nn.Linear.weight)
-  __nv_bfloat16* dst;      // [out, pitch]      K-major operand of the forward GEMM
-  __nv_bfloat16* dst_t;    // [in, pitch_t]     transposed copy: K-major operand of the dgrad GEMM (nullable)
-  int out, in, pitch, pitch_t;
+  __nv_bfloat16* dst;      // [out, pitch]      K-major operand of the forward GEMM, MN-major operand of the dgrad
+  int out, in, pitch;
 };
 
 struct WeightCastGroup {

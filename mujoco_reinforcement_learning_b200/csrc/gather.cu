@@ -13,6 +13,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "tc_ptx.cuh"
 
 namespace b200ppo {
 
@@ -99,10 +100,10 @@ gather_minibatch_tma_kernel(const int64_t* __restrict__ idx, int64_t count, int6
   __shared__ __align__(8) uint64_t bars[32];
   const int lane = threadIdx.x;
   const uint32_t row_bytes = uint32_t(obs_dim) * 4u;
-  const uint32_t slot = static_cast<uint32_t>(__cvta_generic_to_shared(slots)) + lane * row_bytes;
-  const uint32_t bar = static_cast<uint32_t>(__cvta_generic_to_shared(&bars[lane]));
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  const uint32_t slot = smem_u32(slots) + lane * row_bytes;
+  uint64_t* bar = &bars[lane];
+  mbar_init(bar, 1);
+  mbar_init_fence();
   __syncwarp();
   uint32_t phase = 0;
   for (int64_t i = int64_t(blockIdx.x) * 32 + lane; i < count; i += int64_t(gridDim.x) * 32) {
@@ -110,8 +111,8 @@ gather_minibatch_tma_kernel(const int64_t* __restrict__ idx, int64_t count, int6
     const int64_t s = resolve_index(idx, pos, n_rows, err_flag);
     if (s < 0) continue;
     // the previous bulk store of this lane must have finished READING the slot before it is refilled
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(row_bytes) : "memory");
+    bulk_wait_read<0>();
+    mbar_expect_tx(bar, row_bytes);
     const float* src;
     if (parts.count > 0) {
       const int64_t pi = s / parts.rows_per_part;
@@ -119,31 +120,19 @@ gather_minibatch_tma_kernel(const int64_t* __restrict__ idx, int64_t count, int6
     } else {
       src = obs + s * obs_dim;
     }
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(slot), "l"(src),
-                 "r"(row_bytes), "r"(bar)
-                 : "memory");
+    bulk_load(slot, src, row_bytes, bar);
     // short leaves while the row is in flight
     if (act != nullptr)
       for (int k = 0; k < act_dim; ++k) act_o[i * act_dim + k] = __ldg(act + s * act_dim + k);
     if (logp != nullptr) logp_o[i] = __ldg(logp + s);
     if (adv != nullptr) adv_o[i] = __ldg(adv + s);
     if (tgt != nullptr) tgt_o[i] = __ldg(tgt + s);
-    uint32_t done;
-    do {
-      asm volatile(
-          "{\n\t.reg .pred p;\n\t"
-          "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t}"
-          : "=r"(done)
-          : "r"(bar), "r"(phase)
-          : "memory");
-    } while (!done);
+    mbar_wait(bar, phase);
     phase ^= 1u;
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(obs_o + i * obs_dim), "r"(slot), "r"(row_bytes)
-                 : "memory");
-    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+    bulk_store(obs_o + i * obs_dim, slot, row_bytes);
+    bulk_commit();
   }
-  asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+  bulk_wait<0>();
 }
 
 // Same gather, observations emitted as bf16 rows of pitch `pitch` elements with a 1.0 in column obs_dim (the

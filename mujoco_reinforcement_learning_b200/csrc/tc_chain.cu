@@ -59,27 +59,6 @@ static_assert(CH_MISC_B3 + 4 * (kChainMaxAct + 1) <= CH_MISC_CONST && CH_MISC_CO
                   CH_MISC_RED + 16 * CH_RED_W <= CH_MISC_BIAS && CH_MISC_BIAS + 2048 <= CH_MISC,
               "chain kernel misc layout");
 
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {  // arrivals come from the peer CTA too
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-
-// plain bulk copy global -> this CTA's shared memory, bytes counted on a local mbarrier (16-byte granules)
-__device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src), "r"(bytes),
-               "r"(smem_u32(bar))
-               : "memory");
-}
-
 __device__ __forceinline__ void ch_bias16(const float* __restrict__ b, float (&o)[16]) {  // warp-uniform address: one L1 wavefront each
 #pragma unroll
   for (int u = 0; u < 4; ++u) {
@@ -98,16 +77,6 @@ __device__ __forceinline__ void ch_act16(const uint32_t (&v)[16], const float (&
       o[j] = pack_bf16(fmaxf(__uint_as_float(v[2 * j]) + b[2 * j], 0.f), fmaxf(__uint_as_float(v[2 * j + 1]) + b[2 * j + 1], 0.f));
   }
 }
-// 16 bf16 of this thread's row <-> the two swizzled 16-byte units (2s, 2s+1) of its 128-byte tile row
-__device__ __forceinline__ void ch_sts16(uint32_t srow, uint32_t sw, int s, const uint32_t (&o)[8]) {
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(srow + (((2 * s) ^ sw) << 4)), "r"(o[0]), "r"(o[1]), "r"(o[2]), "r"(o[3]) : "memory");
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(srow + (((2 * s + 1) ^ sw) << 4)), "r"(o[4]), "r"(o[5]), "r"(o[6]), "r"(o[7]) : "memory");
-}
-__device__ __forceinline__ void ch_lds16(uint32_t srow, uint32_t sw, int s, uint32_t (&h)[8]) {
-  asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(h[0]), "=r"(h[1]), "=r"(h[2]), "=r"(h[3]) : "r"(srow + (((2 * s) ^ sw) << 4)) : "memory");
-  asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(h[4]), "=r"(h[5]), "=r"(h[6]), "=r"(h[7]) : "r"(srow + (((2 * s + 1) ^ sw) << 4)) : "memory");
-}
-
 __device__ __forceinline__ void ch_lds_bias16(uint32_t saddr, float (&b)[16]) {  // 16 bf16 biases; broadcast reads: every lane the same 32 bytes
 #pragma unroll
   for (int u = 0; u < 2; ++u) {
@@ -129,20 +98,20 @@ __device__ __forceinline__ void ch_epi_forward(uint32_t tcol, uint32_t bias_s, i
   float b[16];
   tmem_ld16_nowait(tcol, va);
   ch_lds_bias16(bias_s, b);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 16, vb);
-  ch_act16(va, b, act, o); ch_sts16(srow, sw, 0, o);
+  ch_act16(va, b, act, o); sts_unit_pair(srow, sw, 0, o);
   ch_lds_bias16(bias_s + 32, b);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 32, va);
-  ch_act16(vb, b, act, o); ch_sts16(srow, sw, 1, o);
+  ch_act16(vb, b, act, o); sts_unit_pair(srow, sw, 1, o);
   ch_lds_bias16(bias_s + 64, b);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 48, vb);
-  ch_act16(va, b, act, o); ch_sts16(srow, sw, 2, o);
+  ch_act16(va, b, act, o); sts_unit_pair(srow, sw, 2, o);
   ch_lds_bias16(bias_s + 96, b);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-  ch_act16(vb, b, act, o); ch_sts16(srow, sw, 3, o);
+  tmem_ld_wait();
+  ch_act16(vb, b, act, o); sts_unit_pair(srow, sw, 3, o);
 }
 
 // dgrad epilogue, activation in shared memory (the tile this thread wrote two steps earlier): dZ = acc * act'(h),
@@ -150,21 +119,21 @@ __device__ __forceinline__ void ch_epi_forward(uint32_t tcol, uint32_t bias_s, i
 __device__ __forceinline__ void ch_epi_dgrad_smem(uint32_t tcol, int act, uint32_t srow, uint32_t sw) {
   uint32_t va[16], vb[16], h[8], o[8];
   tmem_ld16_nowait(tcol, va);
-  ch_lds16(srow, sw, 0, h);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  lds_unit_pair(srow, sw, 0, h);
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 16, vb);
-  ws2_dgrad16(va, h, act, o); ch_sts16(srow, sw, 0, o);
-  ch_lds16(srow, sw, 1, h);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  act_grad16(va, h, act, o); sts_unit_pair(srow, sw, 0, o);
+  lds_unit_pair(srow, sw, 1, h);
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 32, va);
-  ws2_dgrad16(vb, h, act, o); ch_sts16(srow, sw, 1, o);
-  ch_lds16(srow, sw, 2, h);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  act_grad16(vb, h, act, o); sts_unit_pair(srow, sw, 1, o);
+  lds_unit_pair(srow, sw, 2, h);
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 48, vb);
-  ws2_dgrad16(va, h, act, o); ch_sts16(srow, sw, 2, o);
-  ch_lds16(srow, sw, 3, h);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-  ws2_dgrad16(vb, h, act, o); ch_sts16(srow, sw, 3, o);
+  act_grad16(va, h, act, o); sts_unit_pair(srow, sw, 2, o);
+  lds_unit_pair(srow, sw, 3, h);
+  tmem_ld_wait();
+  act_grad16(vb, h, act, o); sts_unit_pair(srow, sw, 3, o);
 }
 
 // dgrad epilogue of the first hidden layer: its activation was overwritten in shared memory by the second layer's, so
@@ -173,20 +142,20 @@ __device__ __forceinline__ void ch_epi_dgrad_smem(uint32_t tcol, int act, uint32
 __device__ __forceinline__ void ch_epi_dgrad_glob(uint32_t tcol, int act, const uint32_t (&ax)[4][8], __nv_bfloat16* grow, bool row_ok) {
   uint32_t va[16], vb[16], o[8];
   tmem_ld16_nowait(tcol, va);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 16, vb);
-  ws2_dgrad16(va, ax[0], act, o);
+  act_grad16(va, ax[0], act, o);
   if (row_ok) stg256(grow, o);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 32, va);
-  ws2_dgrad16(vb, ax[1], act, o);
+  act_grad16(vb, ax[1], act, o);
   if (row_ok) stg256(grow + 16, o);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 48, vb);
-  ws2_dgrad16(va, ax[2], act, o);
+  act_grad16(va, ax[2], act, o);
   if (row_ok) stg256(grow + 32, o);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-  ws2_dgrad16(vb, ax[3], act, o);
+  tmem_ld_wait();
+  act_grad16(vb, ax[3], act, o);
   if (row_ok) stg256(grow + 48, o);
 }
 
@@ -194,38 +163,23 @@ __device__ __forceinline__ void ch_epi_dgrad_glob(uint32_t tcol, int act, const 
 __device__ __forceinline__ void ch_epi_dgrad_stage(uint32_t tcol, int act, const uint32_t (&ax)[4][8], uint32_t srow, uint32_t sw) {
   uint32_t va[16], vb[16], o[8];
   tmem_ld16_nowait(tcol, va);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 16, vb);
-  ws2_dgrad16(va, ax[0], act, o); ch_sts16(srow, sw, 0, o);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  act_grad16(va, ax[0], act, o); sts_unit_pair(srow, sw, 0, o);
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 32, va);
-  ws2_dgrad16(vb, ax[1], act, o); ch_sts16(srow, sw, 1, o);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  act_grad16(vb, ax[1], act, o); sts_unit_pair(srow, sw, 1, o);
+  tmem_ld_wait();
   tmem_ld16_nowait(tcol + 48, vb);
-  ws2_dgrad16(va, ax[2], act, o); ch_sts16(srow, sw, 2, o);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-  ws2_dgrad16(vb, ax[3], act, o); ch_sts16(srow, sw, 3, o);
-}
-
-__device__ __forceinline__ void ldg256_na(const void* p, uint32_t (&r)[8]) {  // coherent 256-bit load that does not linger in L1
-  asm volatile("ld.global.L1::no_allocate.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "l"(p)
-               : "memory");
+  act_grad16(va, ax[2], act, o); sts_unit_pair(srow, sw, 2, o);
+  tmem_ld_wait();
+  act_grad16(vb, ax[3], act, o); sts_unit_pair(srow, sw, 3, o);
 }
 
 __device__ __forceinline__ float ldg_f32_now(const float* p) {  // volatile: issued where it is written, not sunk to its use
   float v;
   asm volatile("ld.global.nc.f32 %0, [%1];" : "=f"(v) : "l"(p));
   return v;
-}
-
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "r"(taddr)
-               : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
 // Sum over the warp's 32 rows of eight per-row values at once: three exchange stages halve the number of values a lane
@@ -306,15 +260,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
     for (int i = 0; i < 18; ++i) mbar_init(&bars[i], 1);
     mbar_init(&epi_done[0], 2 * CH_EPI_WARPS);
     mbar_init(&epi_done[1], 2 * CH_EPI_WARPS);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2, TMEM_COLS>(tmem_slot);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   cluster_sync_all();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   // The observations of a minibatch were gathered before the epoch began — older than the previous kernel — so the
   // producer may request its first tile's X k-blocks while that kernel (the optimizer) is still draining; the weights it
@@ -398,14 +351,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
     }
   } else if (warp == 1) {
     if (lane == 0 && rank == 0) {  // ===== MMA issuer of the pair =====
-      constexpr uint32_t ID_BASE = (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(256 >> 4) << 24);  // D fp32, A/B bf16, M = 256
-      constexpr uint32_t ID_N256 = ID_BASE | (uint32_t(256 >> 3) << 17);
-      constexpr uint32_t ID_N256_BMN = ID_N256 | (1u << 16);
-      constexpr uint32_t ID_N32 = ID_BASE | (uint32_t(32 >> 3) << 17), ID_N16 = ID_BASE | (uint32_t(16 >> 3) << 17);
+      constexpr uint32_t ID_N256 = umma_idesc(256, 256, false, false), ID_N256_BMN = umma_idesc(256, 256, false, true);
+      constexpr uint32_t ID_N32 = umma_idesc(256, 32, false, false), ID_N16 = umma_idesc(256, 16, false, false);
       uint32_t rs = 0, rph = 0, g = 0;
       auto step_begin = [&]() -> uint32_t {  // the epilogue of step g - 2 has drained this accumulator and written this step's A operand
         mbar_wait(&epi_done[g & 1], ((g >> 1) & 1) ^ 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (a.trace != nullptr && blockIdx.x == 0 && g < 60) a.trace[g * 8 + 0] = clock64();
         return tmem_base + (g & 1) * 256u;
       };
@@ -419,7 +370,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
 #endif
       auto ring_wait = [&]() -> uint32_t {
         mbar_wait(&ring_full[rs], rph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
 #ifdef B200PPO_CHAIN_RING_TRACE
         if (a.trace != nullptr && blockIdx.x == 0 && wn < 64) a.trace[480 + wn * 4 + 1] = clock64();
 #endif
@@ -440,7 +391,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
           for (int kb = 0; kb < KB1; ++kb) {
             if (o == 0) {
               mbar_wait(&x_full[kb], uint32_t(ti & 1));
-              asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+              tc_fence_after();
             }
             const uint32_t b = ring_wait(), aa = smem_base + (CH_X0 + kb) * CH_SLOT;
 #pragma unroll
@@ -482,7 +433,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
           const uint32_t d = step_begin();
           if (o == 0) {  // the critic's seeds come from step 5, the previous step (see the note on the order above)
             mbar_wait(&epi_done[1], ((g - 1) >> 1) & 1);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
           }
           const uint32_t b = ring_wait(), aa = smem_base + (o ? CH_DZ3A : CH_DZ3C) * CH_SLOT;
           const int nk = o ? 2 : 1;
@@ -552,7 +503,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
     };
     auto acc_wait = [&]() {
       mbar_wait(&acc_full[g & 1], (g >> 1) & 1);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       __syncwarp();
       tr(2);
     };
@@ -561,18 +512,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
     // part of the next A operand, and the sub-tile it wrote leaves for global memory through the copy engine (one
     // elected lane; rows past the batch are clipped by the tensor map).
     auto step_done = [&](const CUtensorMap* store_map, uint32_t sub, int grow0) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      fence_proxy_async_smem();
+      tc_fence_before();
       __syncwarp();
       if (lane == 0) {
         // relaxed: a release here is MEMBAR.ALL.GPU in front of every arrive (19 % of the first version's stall samples);
         // the proxy fence above has already completed this warp's shared-memory writes, which is all the issuer's MMAs read
-        asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"((g & 1) ? lead_done1 : lead_done0) : "memory");
+        mbar_arrive_cluster((g & 1) ? lead_done1 : lead_done0);
         if (store_map != nullptr) {
-          asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(store_map)),
-                       "r"(sub), "r"(chunk * 64), "r"(grow0)
-                       : "memory");
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          tma_store_2d(store_map, sub, chunk * 64, grow0);
+          bulk_commit();
         }
         if (a.trace != nullptr && blockIdx.x == 0 && g < 60)
           atomicMax(reinterpret_cast<unsigned long long*>(a.trace) + g * 8 + 3, (unsigned long long)clock64());
@@ -585,8 +534,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
     // second youngest elsewhere.
     auto stores_drained = [&](bool youngest) {
       if (lane == 0) {
-        if (youngest) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-        else asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        if (youngest) bulk_wait_read<0>();
+        else bulk_wait_read<1>();
       }
       __syncwarp();
     };
@@ -596,8 +545,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
       if (lane == 0) {
         // (completion of a bulk group makes its writes visible to the waiting thread; __syncwarp orders the other lanes'
         // loads after it.  A fence.proxy.async.global here was measured at ~4 k cycles per use.)
-        if (critic) asm volatile("cp.async.bulk.wait_group 3;" ::: "memory");
-        else asm volatile("cp.async.bulk.wait_group 5;" ::: "memory");
+        if (critic) bulk_wait<3>();
+        else bulk_wait<5>();
       }
       __syncwarp();
     };
@@ -816,19 +765,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
         step_done(&a.net[0].sZ1, sub_a, grow0);
       }
     }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    if (lane == 0) bulk_wait<0>();
     // this CTA's row of loss partials: (sum surrogate, sum huber, sum d loss / d logstd_j)
     asm volatile("bar.sync 1, %0;" ::"n"(CH_EPI_WARPS * 32) : "memory");
     const int t = threadIdx.x - 64;
     if (!INFER && t < 2 + A)
       a.ppo.partials[int64_t(blockIdx.x) * (2 + A) + t] = red_s[t] + red_s[CH_RED_W + t] + red_s[2 * CH_RED_W + t] + red_s[3 * CH_RED_W + t];
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   cluster_sync_all();  // the peer may still be reading this CTA's operands / arriving on its barriers
   if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc<2, TMEM_COLS>(tmem_base);
   }
 }
 

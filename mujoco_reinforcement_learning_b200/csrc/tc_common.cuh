@@ -1,8 +1,10 @@
-// Device-side building blocks shared by the tcgen05 GEMM kernels (tc_gemm.cu, tc_ws.cu).
+// Device-side building blocks shared by the tcgen05 kernels (tc_gemm.cu, tc_persist.cu, tc_ws.cu, tc_wgrad.cu, tc_chain.cu):
+// the one-tile / persistent tile pipeline and the epilogues.  The PTX primitives they are built from live in tc_ptx.cuh.
 #pragma once
 #include <string.h>
 
 #include "tc_gemm.cuh"
+#include "tc_ptx.cuh"
 
 namespace b200ppo {
 
@@ -11,81 +13,6 @@ constexpr int TC_BK = 64;  // bf16 elements: 128 bytes = one swizzle row
 constexpr int TC_EPI_WARPS = 8;                        // two per TMEM lane quarter, each takes half of the columns
 constexpr int TC_THREADS = (2 + TC_EPI_WARPS) * 32;    // + TMA producer warp + MMA issuer warp
 constexpr int TC_A_BYTES = TC_BM * TC_BK * 2;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-// 64-bit shared-memory matrix descriptor (sm_100): 128-byte swizzle, version 1.
-__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= uint64_t((smem_addr & 0x3FFFF) >> 4);
-  d |= uint64_t((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= uint64_t((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= uint64_t(1) << 46;  // descriptor version (Blackwell)
-  d |= uint64_t(2) << 61;  // SWIZZLE_128B
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
 
 // MUFU.TANH: one instruction, max relative error ~2^-11 — below bf16's 2^-8 resolution of the stored activation
 __device__ __forceinline__ float tanh_fast(float x) {
@@ -101,6 +28,87 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 
 __device__ __forceinline__ float split_unscale(float amax_a, float amax_b) {
   return exp2f(float(-(split_exponent(amax_a) + split_exponent(amax_b))));
+}
+
+// ---- tile pipeline of the one-tile (tc_gemm.cu) and persistent (tc_persist.cu) kernels ------------------------------
+// Output tile `tile` of a group: its problem, split-K slice, corner and k range.  n_it ring iterations: in the
+// fp32-tolerance mode the products of the terms run one after the other over the split's k range, smallest terms first.
+struct TcTile {
+  int pi, split, m0, n0, kt_begin, kt_len, n_it;
+};
+
+template <int BN>
+__device__ __forceinline__ TcTile tc_tile(const TcGroup& grp, int tile) {
+  TcTile t;
+  t.pi = 0;
+#pragma unroll 1
+  for (int i = 1; i < grp.count; ++i)
+    if (tile >= grp.p[i].tile_begin) t.pi = i;
+  const TcProblem& P = grp.p[t.pi];
+  int local = tile - P.tile_begin;
+  const int tiles_mn = P.tiles_m * P.tiles_n;
+  t.split = local / tiles_mn;
+  local -= t.split * tiles_mn;
+  t.m0 = (local / P.tiles_n) * TC_BM;
+  t.n0 = (local % P.tiles_n) * BN;
+  const int total_kt = (P.K + TC_BK - 1) / TC_BK;
+  t.kt_begin = t.split * P.k_tiles_per_split;
+  const int kt_end = min(total_kt, t.kt_begin + P.k_tiles_per_split);
+  t.kt_len = max(kt_end - t.kt_begin, 0);
+  t.n_it = P.parts ? split_products(P.parts) * t.kt_len : t.kt_len;
+  return t;
+}
+
+// Producer: the A and B boxes of ring iteration `it` of tile T into one stage, completing on `bar`.
+template <int BN>
+__device__ __forceinline__ void tc_load_stage(const TcProblem& P, const TcTile& T, int it, uint8_t* a, uint8_t* b, uint64_t* bar) {
+  int kb = T.kt_begin + it, ao = 0, bo = 0;  // k tile, offsets of the product's terms along the contiguous dimension
+  if (P.parts) {
+    const int c = it / T.kt_len;
+    kb = T.kt_begin + (it - c * T.kt_len);
+    ao = int((split_terms_a(P.parts) >> (4 * c)) & 3u) * P.a_part;
+    bo = int((split_terms_b(P.parts) >> (4 * c)) & 3u) * P.b_part;
+  }
+  if (!P.a_mn_major) {
+    tma_load_2d(a, &P.tmA, bar, ao + kb * TC_BK, T.m0);
+  } else {
+    tma_load_2d(a, &P.tmA, bar, ao + T.m0, kb * TC_BK);
+    tma_load_2d(a + 64 * TC_BK * 2, &P.tmA, bar, ao + T.m0 + 64, kb * TC_BK);
+  }
+  if (!P.b_mn_major) {
+    tma_load_2d(b, &P.tmB, bar, bo + kb * TC_BK, T.n0);
+  } else {
+#pragma unroll
+    for (int j = 0; j < BN / 64; ++j) tma_load_2d(b + j * 64 * TC_BK * 2, &P.tmB, bar, bo + T.n0 + 64 * j, kb * TC_BK);
+  }
+}
+
+// MMA issuer: a problem's instruction descriptor and operand descriptor steps ...
+struct TcMma {
+  uint32_t idesc, a_lbo, b_lbo, a_kstep, b_kstep;
+};
+
+template <int BN>
+__device__ __forceinline__ TcMma tc_mma_setup(const TcProblem& P) {
+  // K-major SW128: 8-row groups 1024 B apart; one K=16 step = +32 B inside the swizzle row.
+  // MN-major SW128: K atoms (8 k-rows x 128 B) 1024 B apart (SBO), 64-wide MN atoms BK*128 B apart (LBO);
+  //                 one K=16 step = +2048 B.
+  TcMma m;
+  const bool f16 = P.parts == 2;  // operand format: fp16 in the two-term mode, bf16 otherwise
+  m.idesc = umma_idesc(TC_BM, BN, P.a_mn_major != 0, P.b_mn_major != 0, f16);
+  m.a_lbo = P.a_mn_major ? TC_BK * 128 : 0;
+  m.b_lbo = P.b_mn_major ? TC_BK * 128 : 0;
+  m.a_kstep = P.a_mn_major ? 2048 : 32;
+  m.b_kstep = P.b_mn_major ? 2048 : 32;
+  return m;
+}
+
+// ... and the four K = 16 MMAs of one ring stage into the accumulator at TMEM address d
+__device__ __forceinline__ void tc_mma_stage(const TcMma& m, uint32_t d, uint32_t a_addr, uint32_t b_addr, bool accumulate) {
+#pragma unroll
+  for (int k = 0; k < TC_BK / 16; ++k)
+    umma_bf16(d, umma_desc(a_addr + k * m.a_kstep, m.a_lbo, 1024), umma_desc(b_addr + k * m.b_kstep, m.b_lbo, 1024), m.idesc,
+              (accumulate || k > 0) ? 1u : 0u);
 }
 
 // Epilogue of one 128 x BN accumulator tile, executed by the 8 epilogue warps (warp index 2..9 of the CTA).
@@ -161,7 +169,7 @@ __device__ __forceinline__ void tc_epilogue(const TcProblem& P, int split, uint3
     prefetch_aux(c_begin);
     if (has_k) {
       mbar_wait(tmem_full_bar, full_parity);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
     }
 #pragma unroll 1
     for (int c = c_begin; c < c_end; ++c) {
@@ -414,7 +422,7 @@ __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split
   }
   if (has_k) {
     mbar_wait(tmem_full_bar, full_parity);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
   }
   __syncwarp();
   const float* bs = bias_s + col0;
@@ -446,8 +454,7 @@ __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split
       }
     } else {  // TC_EPI_DGRAD: dz = acc * act'(h), h from the staged activation slab (this thread's row)
       uint32_t w[8];
-      asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]) : "r"(my_row + uint32_t(((2 * s) ^ sw) << 4)) : "memory");
-      asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7]) : "r"(my_row + uint32_t(((2 * s + 1) ^ sw) << 4)) : "memory");
+      lds_unit_pair(my_row, sw, s, w);
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const __nv_bfloat162 b2 = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
@@ -457,17 +464,14 @@ __device__ __forceinline__ void tc_epilogue_staged(const TcProblem& P, int split
         else o[j] = pack_bf16(h0 > 0.f ? g0 : 0.f, h1 > 0.f ? g1 : 0.f);
       }
     }
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(my_row + uint32_t(((2 * s) ^ sw) << 4)), "r"(o[0]), "r"(o[1]), "r"(o[2]), "r"(o[3]) : "memory");
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(my_row + uint32_t(((2 * s + 1) ^ sw) << 4)), "r"(o[4]), "r"(o[5]), "r"(o[6]), "r"(o[7]) : "memory");
+    sts_unit_pair(my_row, sw, s, o);
   }
   if constexpr (TMA_OUT) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy st.shared -> visible to the copy engine
+    fence_proxy_async_smem();  // generic-proxy st.shared -> visible to the copy engine
     __syncwarp();
     if (lane == 0) {  // rows >= M and columns >= N are clipped by the tensor map
-      asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(tm_out)),
-                   "r"(sbase), "r"(n0 + col0), "r"(mq)
-                   : "memory");
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+      tma_store_2d(tm_out, sbase, n0 + col0, mq);
+      bulk_commit();
     }
     return;
   }
@@ -649,7 +653,7 @@ __device__ __forceinline__ void tc_epilogue_ppo(const TcProblem& P, uint32_t tme
     else tgt = __ldg(P.ppo.target + m);
   }
   mbar_wait(tmem_full_bar, full_parity);
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   __syncwarp();
   if (!worker) return;
   if (P.epilogue == TC_EPI_PPO_CRITIC) {
@@ -729,57 +733,8 @@ __device__ __forceinline__ void tc_ppo_finish(const TcProblem& P, int warp, int 
   }
 }
 
-// ---- CTA-pair (cta_group::2) building blocks shared by tc_ws.cu and tc_chain.cu ---------------------------------------------
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA load whose completion bytes are counted on an mbarrier of the pair's leader CTA (shared::cluster address)
-__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma2_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma2_commit(uint64_t* bar) {  // arrives on the barrier at this offset in BOTH CTAs
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(uint16_t(3))
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr)
-      : "memory");
-}
-
-// 16 accumulator columns of this thread's row -> bias + activation -> bf16 -> two swizzled 16-byte units of the row
 // 16 accumulator columns of this thread's row -> bias + activation -> 16 bf16 (8 words)
-__device__ __forceinline__ void ws2_act16(const uint32_t (&v)[16], const float* bs, int act, uint32_t (&o)[8]) {
+__device__ __forceinline__ void bias_act16(const uint32_t (&v)[16], const float* bs, int act, uint32_t (&o)[8]) {
   float z[16];
 #pragma unroll
   for (int u = 0; u < 4; ++u) {
@@ -798,26 +753,12 @@ __device__ __forceinline__ void ws2_act16(const uint32_t (&v)[16], const float* 
 // ... into two swizzled 16-byte units of the row's staging line
 __device__ __forceinline__ void ws2_finish16(const uint32_t (&v)[16], const float* bs, int act, uint32_t my_row, int sw, int s) {
   uint32_t o[8];
-  ws2_act16(v, bs, act, o);
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(my_row + uint32_t(((2 * s) ^ sw) << 4)), "r"(o[0]), "r"(o[1]), "r"(o[2]), "r"(o[3]) : "memory");
-  asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(my_row + uint32_t(((2 * s + 1) ^ sw) << 4)), "r"(o[4]), "r"(o[5]), "r"(o[6]), "r"(o[7]) : "memory");
+  bias_act16(v, bs, act, o);
+  sts_unit_pair(my_row, sw, s, o);
 }
 
-// 256-bit global accesses (one full 32-byte sector per thread): the dgrad epilogue of the pair kernel reads its
-// activation row and writes its result row straight from registers — no staging tile, so shared memory is left to the
-// operands (W half + a deep A ring) and the epilogue does not compete with the MMAs for shared-memory bandwidth.
-__device__ __forceinline__ void ldg256(const void* p, uint32_t (&r)[8]) {
-  asm volatile("ld.global.nc.L1::no_allocate.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "l"(p));
-}
-__device__ __forceinline__ void stg256(void* p, const uint32_t (&r)[8]) {
-  asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]),
-               "r"(r[5]), "r"(r[6]), "r"(r[7])
-               : "memory");
-}
 // dz = acc * act'(h) for 16 columns of this thread's row; h: 16 bf16 activations (8 words)
-__device__ __forceinline__ void ws2_dgrad16(const uint32_t (&v)[16], const uint32_t (&h)[8], int act, uint32_t (&o)[8]) {
+__device__ __forceinline__ void act_grad16(const uint32_t (&v)[16], const uint32_t (&h)[8], int act, uint32_t (&o)[8]) {
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
     const float h0 = __uint_as_float(h[j] << 16), h1 = __uint_as_float(h[j] & 0xFFFF0000u);

@@ -13,9 +13,8 @@
 //                          splitting the columns), fused bias + MUFU tanh / relu, or
 //                          activation-derivative multiply (dgrad), or fp32 split-K partial store (wgrad) with
 //                          the bias gradient read off an appended ones-column of the B operand.
-// Operands may be K-major or MN-major (UMMA descriptor major bits), so forward (X W^T), dgrad (dZ W via a
-// transposed bf16 weight copy) and wgrad (dZ^T X, both operands MN-major) share the kernel with no transposes
-// of activations.
+// Operands may be K-major or MN-major (UMMA descriptor major bits), so forward (X W^T), dgrad (dZ W, W MN-major)
+// and wgrad (dZ^T X, both operands MN-major) share the kernel with no transposes.
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -66,23 +65,10 @@ __global__ void __launch_bounds__(TC_THREADS, OCC) tc_gemm_kernel(const __grid_c
     trc[7] = smid;
   }
 
-  int pi = 0;
-#pragma unroll 1
-  for (int i = 1; i < grp.count; ++i)
-    if (int(blockIdx.x) >= grp.p[i].tile_begin) pi = i;
-  const TcProblem& P = grp.p[pi];
-  int local = int(blockIdx.x) - P.tile_begin;
-  const int tiles_mn = P.tiles_m * P.tiles_n;
-  const int split = local / tiles_mn;
-  local -= split * tiles_mn;
-  const int m0 = (local / P.tiles_n) * TC_BM, n0 = (local % P.tiles_n) * BN;
-  const int total_kt = (P.K + TC_BK - 1) / TC_BK;
-  const int kt_begin = split * P.k_tiles_per_split;
-  const int kt_end = min(total_kt, kt_begin + P.k_tiles_per_split);
-  const bool has_k = kt_end > kt_begin;
-  // fp32-tolerance mode: the six products run one after the other over this split's k range, smallest terms first
-  const int kt_len = kt_end - kt_begin;
-  const int n_it = P.parts ? split_products(P.parts) * kt_len : kt_len;
+  const TcTile T = tc_tile<BN>(grp, int(blockIdx.x));
+  const TcProblem& P = grp.p[T.pi];
+  const int split = T.split, m0 = T.m0, n0 = T.n0, n_it = T.n_it;
+  const bool has_k = n_it > 0;
 
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < TC_STAGES; ++s) {
@@ -90,14 +76,13 @@ __global__ void __launch_bounds__(TC_THREADS, OCC) tc_gemm_kernel(const __grid_c
       mbar_init(&empty_bar[s], 1);
     }
     mbar_init(tmem_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1, TMEM_COLS>(tmem_slot);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait_then_release();  // everything below reads what earlier kernels of the chain wrote
   if (trc != nullptr && threadIdx.x == 0) trc[1] = clock64();
@@ -114,54 +99,21 @@ __global__ void __launch_bounds__(TC_THREADS, OCC) tc_gemm_kernel(const __grid_c
         const uint32_t ph = (it / TC_STAGES) & 1;
         mbar_wait(&empty_bar[s], ph ^ 1);
         mbar_expect_tx(&full_bar[s], TC_A_BYTES + B_BYTES);
-        uint8_t* a = sA + s * TC_A_BYTES;
-        uint8_t* b = sB + s * B_BYTES;
-        int kb = kt_begin + it, ao = 0, bo = 0;  // k tile, offsets of the product's terms along the contiguous dimension
-        if (P.parts) {
-          const int c = it / kt_len;
-          kb = kt_begin + (it - c * kt_len);
-          ao = int((split_terms_a(P.parts) >> (4 * c)) & 3u) * P.a_part;
-          bo = int((split_terms_b(P.parts) >> (4 * c)) & 3u) * P.b_part;
-        }
-        if (!P.a_mn_major) {
-          tma_load_2d(a, &P.tmA, &full_bar[s], ao + kb * TC_BK, m0);
-        } else {
-          tma_load_2d(a, &P.tmA, &full_bar[s], ao + m0, kb * TC_BK);
-          tma_load_2d(a + 64 * TC_BK * 2, &P.tmA, &full_bar[s], ao + m0 + 64, kb * TC_BK);
-        }
-        if (!P.b_mn_major) {
-          tma_load_2d(b, &P.tmB, &full_bar[s], bo + kb * TC_BK, n0);
-        } else {
-#pragma unroll
-          for (int j = 0; j < BN / 64; ++j) tma_load_2d(b + j * 64 * TC_BK * 2, &P.tmB, &full_bar[s], bo + n0 + 64 * j, kb * TC_BK);
-        }
+        tc_load_stage<BN>(P, T, it, sA + s * TC_A_BYTES, sB + s * B_BYTES, &full_bar[s]);
       }
     }
   } else if (warp == 1) {
     if (has_k) {  // ===== MMA issuer =====
-      // instruction descriptor: D fp32, A/B bf16, majors, N>>3, M>>4
-      const uint32_t fmt = P.parts == 2 ? 0u : 1u;  // operand format: F16 for the two-term mode, BF16 otherwise
-      const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (uint32_t(P.a_mn_major != 0) << 15) |
-                             (uint32_t(P.b_mn_major != 0) << 16) | (uint32_t(BN >> 3) << 17) | (uint32_t(TC_BM >> 4) << 24);
-      // K-major SW128: 8-row groups 1024 B apart; one K=16 step = +32 B inside the swizzle row.
-      // MN-major SW128: K atoms (8 k-rows x 128 B) 1024 B apart (SBO), 64-wide MN atoms BK*128 B apart (LBO);
-      //                 one K=16 step = +2048 B.
-      const uint32_t a_lbo = P.a_mn_major ? TC_BK * 128 : 0, b_lbo = P.b_mn_major ? TC_BK * 128 : 0;
-      const uint32_t a_kstep = P.a_mn_major ? 2048 : 32, b_kstep = P.b_mn_major ? 2048 : 32;
+      const TcMma mma = tc_mma_setup<BN>(P);
       for (int it = 0; it < n_it; ++it) {
         const int s = it % TC_STAGES;
         const uint32_t ph = (it / TC_STAGES) & 1;
         mbar_wait(&full_bar[s], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (trc != nullptr && lane == 0 && it == 0) trc[2] = clock64();
         if (trc != nullptr && lane == 0 && it == n_it - 1) trc[3] = clock64();
         if (lane == 0) {
-          const uint32_t a_addr = smem_u32(sA + s * TC_A_BYTES), b_addr = smem_u32(sB + s * B_BYTES);
-#pragma unroll
-          for (int k = 0; k < TC_BK / 16; ++k) {
-            umma_bf16(tmem_base, umma_desc(a_addr + k * a_kstep, a_lbo, 1024), umma_desc(b_addr + k * b_kstep, b_lbo, 1024),
-                      idesc, (it > 0 || k > 0) ? 1u : 0u);
-          }
+          tc_mma_stage(mma, tmem_base, smem_u32(sA + s * TC_A_BYTES), smem_u32(sB + s * B_BYTES), it > 0);
           umma_commit(&empty_bar[s]);
           if (it == n_it - 1) umma_commit(tmem_full_bar);
         }
@@ -186,14 +138,14 @@ __global__ void __launch_bounds__(TC_THREADS, OCC) tc_gemm_kernel(const __grid_c
         tc_epilogue<BN>(P, split, tmem_base, has_k, m0, n0, warp, lane, tmem_full_bar, 0, bias_s);
       }
     } else tc_epilogue<BN>(P, split, tmem_base, has_k, m0, n0, warp, lane, tmem_full_bar, 0, bias_s);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     if (trc != nullptr && warp == 2 && lane == 0) trc[5] = clock64();
   }
   __syncthreads();
   if (trc != nullptr && threadIdx.x == 0) trc[6] = clock64();
   if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc<1, TMEM_COLS>(tmem_base);
   }
 }
 

@@ -21,32 +21,6 @@ template <int BN> struct PersistCfg {
   static constexpr int STAGES = BN <= 192 ? 5 : 4;  // 200 / 192 KB of operands
 };
 
-struct PersistTile {
-  int pi, split, m0, n0, kt_begin, kt_len, n_it;
-};
-
-template <int BN>
-__device__ __forceinline__ PersistTile persist_tile(const TcGroup& grp, int tile) {
-  PersistTile t;
-  t.pi = 0;
-#pragma unroll 1
-  for (int i = 1; i < grp.count; ++i)
-    if (tile >= grp.p[i].tile_begin) t.pi = i;
-  const TcProblem& P = grp.p[t.pi];
-  int local = tile - P.tile_begin;
-  const int tiles_mn = P.tiles_m * P.tiles_n;
-  t.split = local / tiles_mn;
-  local -= t.split * tiles_mn;
-  t.m0 = (local / P.tiles_n) * TC_BM;
-  t.n0 = (local % P.tiles_n) * BN;
-  const int total_kt = (P.K + TC_BK - 1) / TC_BK;
-  t.kt_begin = t.split * P.k_tiles_per_split;
-  const int kt_end = min(total_kt, t.kt_begin + P.k_tiles_per_split);
-  t.kt_len = max(kt_end - t.kt_begin, 0);
-  t.n_it = P.parts ? split_products(P.parts) * t.kt_len : t.kt_len;
-  return t;
-}
-
 template <int BN>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_persist_kernel(const __grid_constant__ TcGroup grp) {
   constexpr int STAGES = PersistCfg<BN>::STAGES;
@@ -74,14 +48,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_persist_kernel(const __grid_
       mbar_init(&acc_full[i], 1);
       mbar_init(&acc_empty[i], TC_EPI_WARPS);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1, TMEM_COLS>(tmem_slot);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait_then_release();  // everything below reads what earlier kernels of the stream wrote
 
@@ -93,64 +66,36 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_persist_kernel(const __grid_
     if (lane == 0) {  // ===== TMA producer =====
       uint32_t git = 0;  // ring iterations since the kernel began
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const PersistTile T = persist_tile<BN>(grp, tile);
+        const TcTile T = tc_tile<BN>(grp, tile);
         const TcProblem& P = grp.p[T.pi];
         for (int it = 0; it < T.n_it; ++it, ++git) {
           const uint32_t s = git % STAGES, ph = (git / STAGES) & 1;
           mbar_wait(&empty_bar[s], ph ^ 1);
           if (trc != nullptr && tile / int(gridDim.x) < 64 && (it == 0 || it == T.n_it - 1)) trc[(tile / gridDim.x) * 8 + (it == 0 ? 5 : 6)] = clock64();
           mbar_expect_tx(&full_bar[s], TC_A_BYTES + B_BYTES);
-          uint8_t* a = sA + s * TC_A_BYTES;
-          uint8_t* b = sB + s * B_BYTES;
-          int kb = T.kt_begin + it, ao = 0, bo = 0;
-          if (P.parts) {
-            const int c = it / T.kt_len;
-            kb = T.kt_begin + (it - c * T.kt_len);
-            ao = int((split_terms_a(P.parts) >> (4 * c)) & 3u) * P.a_part;
-            bo = int((split_terms_b(P.parts) >> (4 * c)) & 3u) * P.b_part;
-          }
-          if (!P.a_mn_major) {
-            tma_load_2d(a, &P.tmA, &full_bar[s], ao + kb * TC_BK, T.m0);
-          } else {
-            tma_load_2d(a, &P.tmA, &full_bar[s], ao + T.m0, kb * TC_BK);
-            tma_load_2d(a + 64 * TC_BK * 2, &P.tmA, &full_bar[s], ao + T.m0 + 64, kb * TC_BK);
-          }
-          if (!P.b_mn_major) {
-            tma_load_2d(b, &P.tmB, &full_bar[s], bo + kb * TC_BK, T.n0);
-          } else {
-#pragma unroll
-            for (int j = 0; j < BN / 64; ++j) tma_load_2d(b + j * 64 * TC_BK * 2, &P.tmB, &full_bar[s], bo + T.n0 + 64 * j, kb * TC_BK);
-          }
+          tc_load_stage<BN>(P, T, it, sA + s * TC_A_BYTES, sB + s * B_BYTES, &full_bar[s]);
         }
       }
     }
   } else if (warp == 1) {  // ===== MMA issuer =====
     uint32_t git = 0, use = 0;  // ring iterations; accumulators handed out so far
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const PersistTile T = persist_tile<BN>(grp, tile);
+      const TcTile T = tc_tile<BN>(grp, tile);
       if (T.n_it <= 0) continue;
       const TcProblem& P = grp.p[T.pi];
       const uint32_t acc = use & 1;
       mbar_wait(&acc_empty[acc], ((use >> 1) & 1) ^ 1);  // the epilogue drained this accumulator (two uses ago)
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       if (trc != nullptr && lane == 0 && tile / int(gridDim.x) < 64) trc[(tile / gridDim.x) * 8 + 0] = clock64();
       const uint32_t d = tmem_base + acc * ACC_STRIDE;
-      const uint32_t fmt = P.parts == 2 ? 0u : 1u;  // operand format: F16 for the two-term mode, BF16 otherwise
-      const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (uint32_t(P.a_mn_major != 0) << 15) |
-                             (uint32_t(P.b_mn_major != 0) << 16) | (uint32_t(BN >> 3) << 17) | (uint32_t(TC_BM >> 4) << 24);
-      const uint32_t a_lbo = P.a_mn_major ? TC_BK * 128 : 0, b_lbo = P.b_mn_major ? TC_BK * 128 : 0;
-      const uint32_t a_kstep = P.a_mn_major ? 2048 : 32, b_kstep = P.b_mn_major ? 2048 : 32;
+      const TcMma mma = tc_mma_setup<BN>(P);
       for (int it = 0; it < T.n_it; ++it, ++git) {
         const uint32_t s = git % STAGES, ph = (git / STAGES) & 1;
         mbar_wait(&full_bar[s], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (trc != nullptr && lane == 0 && tile / int(gridDim.x) < 64 && (it == 0 || it == T.n_it - 1)) trc[(tile / gridDim.x) * 8 + (it == 0 ? 1 : 2)] = clock64();
         if (lane == 0) {
-          const uint32_t a_addr = smem_u32(sA + s * TC_A_BYTES), b_addr = smem_u32(sB + s * B_BYTES);
-#pragma unroll
-          for (int k = 0; k < TC_BK / 16; ++k)
-            umma_bf16(d, umma_desc(a_addr + k * a_kstep, a_lbo, 1024), umma_desc(b_addr + k * b_kstep, b_lbo, 1024), idesc,
-                      (it > 0 || k > 0) ? 1u : 0u);
+          tc_mma_stage(mma, d, smem_u32(sA + s * TC_A_BYTES), smem_u32(sB + s * B_BYTES), it > 0);
           umma_commit(&empty_bar[s]);
           if (it == T.n_it - 1) umma_commit(&acc_full[acc]);
         }
@@ -161,7 +106,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_persist_kernel(const __grid_
   } else {  // ===== epilogue warps 2..9 =====
     uint32_t use = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const PersistTile T = persist_tile<BN>(grp, tile);
+      const TcTile T = tc_tile<BN>(grp, tile);
       const TcProblem& P = grp.p[T.pi];
       const bool has_k = T.n_it > 0;
       const uint32_t acc = use & 1;
@@ -174,18 +119,18 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_persist_kernel(const __grid_
       tc_epilogue<BN, true>(P, T.split, tmem_base + acc * ACC_STRIDE, has_k, T.m0, T.n0, warp, lane, &acc_full[acc], (use >> 1) & 1, bs);
       if (trc != nullptr && warp == 2 && lane == 0 && tile / int(gridDim.x) < 64) trc[(tile / gridDim.x) * 8 + 4] = clock64();
       if (has_k) {
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_empty[acc]);
         ++use;
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc<1, TMEM_COLS>(tmem_base);
   }
 }
 

@@ -40,40 +40,6 @@ struct Wg2Group {
   int count, n_tiles, max_splits;  // max_splits: partial slots the consumer sums; blocks with fewer splits zero-fill the rest
 };
 
-__device__ __forceinline__ uint32_t wg2_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t wg2_mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void wg2_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void wg2_tma_pair(void* dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void wg2_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void wg2_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(uint16_t(3))
-               : "memory");
-}
-
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) tc_wgrad2_kernel(const __grid_constant__ Wg2Group grp) {
   constexpr uint32_t TMEM_COLS = 512;
   constexpr uint32_t BIAS_COL = 256;  // TMEM column of the 32-wide bias accumulator
@@ -88,7 +54,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) tc_wg
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(done_bar + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = wg2_ctarank();
+  const uint32_t rank = cluster_ctarank();
   const int pair = int(blockIdx.x) >> 1;
   int ti = 0;
 #pragma unroll 1
@@ -106,19 +72,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) tc_wg
 
   // constant B operand of the bias MMA: bf16 ones (any layout of ones is a tile of ones)
   for (int i = threadIdx.x; i < WG2_ONES_BYTES / 4; i += TC_THREADS) reinterpret_cast<uint32_t*>(ones)[i] = 0x3F803F80u;
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  fence_proxy_async_smem();
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < WG2_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     mbar_init(done_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2, TMEM_COLS>(tmem_slot);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  wg2_cluster_sync();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  cluster_sync_all();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait_then_release();  // dZ and H come from the kernels before this one
 
@@ -131,39 +96,38 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) tc_wg
         const uint32_t ph = (it / WG2_STAGES) & 1;
         mbar_wait(&empty_bar[s], ph ^ 1);
         if (rank == 0) mbar_expect_tx(&full_bar[s], stage_tx);
-        const uint32_t leader_full = wg2_mapa(smem_u32(&full_bar[s]), 0);
+        const uint32_t leader_full = mapa_u32(smem_u32(&full_bar[s]), 0);
         uint8_t* a = ring + s * WG2_STAGE_BYTES;
         uint8_t* b = a + TC_A_BYTES;
-        wg2_tma_pair(a, &P.tmA, leader_full, ma, kt * TC_BK);
-        wg2_tma_pair(a + 64 * TC_BK * 2, &P.tmA, leader_full, ma + 64, kt * TC_BK);
-        wg2_tma_pair(b, &P.tmB, leader_full, nb, kt * TC_BK);
-        if (nw_half > 64) wg2_tma_pair(b + 64 * TC_BK * 2, &P.tmB, leader_full, nb + 64, kt * TC_BK);
+        tma_load_2d_pair(a, &P.tmA, leader_full, ma, kt * TC_BK);
+        tma_load_2d_pair(a + 64 * TC_BK * 2, &P.tmA, leader_full, ma + 64, kt * TC_BK);
+        tma_load_2d_pair(b, &P.tmB, leader_full, nb, kt * TC_BK);
+        if (nw_half > 64) tma_load_2d_pair(b + 64 * TC_BK * 2, &P.tmB, leader_full, nb + 64, kt * TC_BK);
       }
     }
   } else if (warp == 1) {
     if (lane == 0 && rank == 0 && has_k) {  // ===== MMA issuer of the pair =====
       // D fp32, A/B bf16, both MN-major, N = nw, M = 256 | bias: B K-major (ones), N = 32
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | (uint32_t(T.nw >> 3) << 17) |
-                             (uint32_t((2 * TC_BM) >> 4) << 24);
-      const uint32_t idesc_bias = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (uint32_t(32 >> 3) << 17) | (uint32_t((2 * TC_BM) >> 4) << 24);
+      const uint32_t idesc = umma_idesc(2 * TC_BM, T.nw, true, true);
+      constexpr uint32_t idesc_bias = umma_idesc(2 * TC_BM, 32, true, false);
       const uint32_t lbo = TC_BK * 128;  // 64-wide MN atoms are 8 KB apart; a K = 16 step is 16 rows of 128 B
       const uint32_t ones_addr = smem_u32(ones);
       for (int kt = kt_begin, it = 0; kt < kt_end; ++kt, ++it) {
         const int s = it % WG2_STAGES;
         const uint32_t ph = (it / WG2_STAGES) & 1;
         mbar_wait(&full_bar[s], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t a_addr = smem_u32(ring + s * WG2_STAGE_BYTES), b_addr = a_addr + TC_A_BYTES;
 #pragma unroll
         for (int k = 0; k < TC_BK / 16; ++k) {
           const uint64_t ad = umma_desc(a_addr + k * 2048, lbo, 1024);
           const uint32_t acc = (it > 0 || k > 0) ? 1u : 0u;
-          wg2_mma(tmem_base, ad, umma_desc(b_addr + k * 2048, lbo, 1024), idesc, acc);
-          if (T.bias) wg2_mma(tmem_base + BIAS_COL, ad, umma_desc(ones_addr + k * 32, 0, 1024), idesc_bias, acc);
+          umma2_bf16(tmem_base, ad, umma_desc(b_addr + k * 2048, lbo, 1024), idesc, acc);
+          if (T.bias) umma2_bf16(tmem_base + BIAS_COL, ad, umma_desc(ones_addr + k * 32, 0, 1024), idesc_bias, acc);
         }
-        wg2_commit(&empty_bar[s]);
+        umma2_commit(&empty_bar[s]);
       }
-      wg2_commit(done_bar);
+      umma2_commit(done_bar);
     }
   } else {  // ===== epilogue: fp32 partials of this CTA's 128 rows =====
     const int q = warp & 3, half = (warp - 2) >> 2;
@@ -171,7 +135,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) tc_wg
     const bool row_ok = m < P.M;
     if (has_k) {
       mbar_wait(done_bar, 0);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
     }
     float* outp = P.out_f32 + int64_t(split) * P.split_stride + int64_t(m) * P.ld_f32;
     const bool vec = (P.ld_f32 % 4 == 0) && (P.split_stride % 4 == 0) && ((reinterpret_cast<uintptr_t>(P.out_f32) & 15u) == 0);
@@ -220,13 +184,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) tc_wg
       }
       if (T.bias && half == 0 && P.bias_grad != nullptr) P.bias_grad[int64_t(z) * P.split_stride + m] = 0.f;
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
   }
   __syncthreads();
-  wg2_cluster_sync();  // the peer's MMAs read this CTA's operands until the last commit
+  cluster_sync_all();  // the peer's MMAs read this CTA's operands until the last commit
   if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc<2, TMEM_COLS>(tmem_base);
   }
 }
 

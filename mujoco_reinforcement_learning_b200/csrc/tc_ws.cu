@@ -69,14 +69,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
     // fused PPO epilogue: the two warp groups alternate tiles, so only four warps release an accumulator
     const uint32_t releasers = P.epilogue >= TC_EPI_PPO_ACTOR ? TC_EPI_WARPS / 2 : TC_EPI_WARPS;
     for (int b = 0; b < 2; ++b) { mbar_init(&acc_full[b], 1); mbar_init(&acc_empty[b], releasers); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1, TMEM_COLS>(tmem_slot);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   auto load_w = [&]() {
@@ -114,20 +113,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
     }
   } else if (warp == 1) {  // ===== MMA issuer: ONE thread runs the whole loop (31 idle lanes would only add polling) =====
     if (lane == 0) {
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(P.b_mn_major != 0) << 16) | (uint32_t(BN >> 3) << 17) |
-                             (uint32_t(TC_BM >> 4) << 24);
+      const uint32_t idesc = umma_idesc(TC_BM, BN, false, P.b_mn_major != 0);
       const uint32_t b_lbo = P.b_mn_major ? TC_BK * 128 : 0, b_kstep = P.b_mn_major ? 2048 : 32;
       mbar_wait(w_full, 0);
       int it = 0, t = 0;
       for (int tile = cta_local; tile < tiles_m; tile += ctas, ++t) {
         const int buf = t & 1;
         mbar_wait(&acc_empty[buf], ((t >> 1) & 1) ^ 1);  // epilogue has drained this accumulator
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         for (int kb = 0; kb < KB; ++kb, ++it) {
           const int s = it % a_stages;
           const uint32_t ph = (it / a_stages) & 1;
           mbar_wait(&a_full[s], ph);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t a_addr = smem_u32(sA + size_t(s) * TC_A_BYTES), b_addr = smem_u32(sW + size_t(kb) * W_KB_BYTES);
 #pragma unroll
           for (int k = 0; k < TC_BK / 16; ++k)
@@ -158,7 +156,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
           tc_ppo_issue(P, next * TC_BM, warp, lane, st[(u & 1) ^ 1], next < tiles_m);
           tc_epilogue_ppo<BN>(P, tmem_base + uint32_t(grp_id * BN), tile * TC_BM, warp, lane, &acc_full[grp_id], uint32_t(u & 1),
                               st[u & 1], bias_s, consts_s, 1, acc, true);
-          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+          tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(&acc_empty[grp_id]);
         }
@@ -182,8 +180,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
           if (tma_out) {
             // tile `cur` was last read by the bulk store of row tile t - ntiles, `nxt` by that of t + 1 - ntiles
             if (lane == 0) {
-              if (ntiles == 1 || (ntiles == 2 && P.epilogue == TC_EPI_DGRAD)) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-              else asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+              if (ntiles == 1 || (ntiles == 2 && P.epilogue == TC_EPI_DGRAD)) bulk_wait_read<0>();
+              else bulk_wait_read<1>();
             }
             __syncwarp();
           }
@@ -198,28 +196,28 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_ws_kernel(const __grid_const
         } else {
           tc_epilogue<BN>(P, 0, tmem_base + uint32_t(buf * BN), true, tile * TC_BM, n0, warp, lane, &acc_full[buf], uint32_t((t >> 1) & 1), bias_s);
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_empty[buf]);
       }
-      if (tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+      if (tma_out && lane == 0) bulk_wait<0>();
       asm volatile("cp.async.wait_group 0;" ::: "memory");
       }
     } else {
       for (int tile = cta_local; tile < tiles_m; tile += ctas, ++t) {
         const int buf = t & 1;
         tc_epilogue<BN>(P, 0, tmem_base + uint32_t(buf * BN), true, tile * TC_BM, n0, warp, lane, &acc_full[buf], uint32_t((t >> 1) & 1), bias_s);
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_empty[buf]);
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc<1, TMEM_COLS>(tmem_base);
   }
 }
 
@@ -276,15 +274,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
     for (int kb = 0; kb < KB; ++kb) mbar_init(&w_full[kb], 1);
     for (int s = 0; s < a_stages; ++s) { mbar_init(&a_full[s], 1); mbar_init(&a_empty[s], 1); }
     for (int b = 0; b < 2; ++b) { mbar_init(&acc_full[b], 1); mbar_init(&acc_empty[b], 2 * WS2_EPI_WARPS); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   } else if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2, TMEM_COLS>(tmem_slot);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   cluster_sync_all();  // both CTAs' barriers exist before any remote arrive / TMA completion targets them
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const bool w_early = grp.w_early != 0;
   if (!(warp == 0 && lane == 0 && w_early)) pdl_wait_then_release();  // the producer lane first requests W (below)
@@ -326,20 +323,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
     }
   } else if (warp == 1) {
     if (lane == 0 && rank == 0) {  // ===== MMA issuer of the pair =====
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(P.b_mn_major != 0) << 16) | (uint32_t(BN >> 3) << 17) |
-                             (uint32_t((2 * TC_BM) >> 4) << 24);
+      const uint32_t idesc = umma_idesc(2 * TC_BM, BN, false, P.b_mn_major != 0);
       const uint32_t b_lbo = P.b_mn_major ? TC_BK * 128 : 0, b_kstep = P.b_mn_major ? 2048 : 32;
       int it = 0, t = 0;
       for (int tile = pair_local; tile < tiles2; tile += pairs, ++t) {
         const int buf = t & 1;
         mbar_wait(&acc_empty[buf], ((t >> 1) & 1) ^ 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         for (int kb = 0; kb < KB; ++kb, ++it) {
           const int s = it % a_stages;
           const uint32_t ph = (it / a_stages) & 1;
           if (t == 0) mbar_wait(&w_full[kb], 0);
           mbar_wait(&a_full[s], ph);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t a_addr = smem_u32(sA + size_t(s) * TC_A_BYTES), b_addr = smem_u32(sW + size_t(kb) * W_KB_BYTES);
 #pragma unroll
           for (int k = 0; k < TC_BK / 16; ++k)
@@ -362,6 +358,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
     const int col0 = chunk * 64;
     const float* bs = bias_s + col0;
     int t = 0, tile_i = 0;
+    // dgrad straight from registers, no staging tile: shared memory is left to the operands (W half + a deep A ring), and
+    // the epilogue does not compete with the MMAs for shared-memory bandwidth
     if (P.epilogue == TC_EPI_DGRAD) {  // direct: activation row in, result row out, 32 bytes per access (rows are 32-byte aligned)
       const bool cols_ok = n0 + col0 + 64 <= P.N;
       for (int tile = pair_local; tile < tiles2; tile += pairs, ++t) {
@@ -387,7 +385,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
         }
         const uint32_t tcol = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(buf * BN + col0);
         mbar_wait(&acc_full[buf], uint32_t((t >> 1) & 1));
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         __syncwarp();
         uint32_t va[16], vb[16], o[8];
         auto emit = [&](int sidx) {
@@ -404,20 +402,20 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
           }
         };
         tmem_ld16_nowait(tcol, va);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld_wait();
         tmem_ld16_nowait(tcol + 16, vb);
-        ws2_dgrad16(va, ax[0], act, o); emit(0);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        act_grad16(va, ax[0], act, o); emit(0);
+        tmem_ld_wait();
         tmem_ld16_nowait(tcol + 32, va);
-        ws2_dgrad16(vb, ax[1], act, o); emit(1);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        act_grad16(vb, ax[1], act, o); emit(1);
+        tmem_ld_wait();
         tmem_ld16_nowait(tcol + 48, vb);
-        ws2_dgrad16(va, ax[2], act, o); emit(2);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        act_grad16(va, ax[2], act, o); emit(2);
+        tmem_ld_wait();
+        tc_fence_before();
         __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(buf ? leader_empty1 : leader_empty0) : "memory");
-        ws2_dgrad16(vb, ax[3], act, o); emit(3);
+        if (lane == 0) mbar_arrive_cluster(buf ? leader_empty1 : leader_empty0);
+        act_grad16(vb, ax[3], act, o); emit(3);
       }
     } else if (grp.tma_out[pidx] == 0) {  // forward, direct: 32-byte row segments from registers (rows 32-byte aligned, whole chunk < N)
       for (int tile = pair_local; tile < tiles2; tile += pairs, ++t) {
@@ -427,27 +425,27 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
         __nv_bfloat16* orow = P.out_bf16 + int64_t(row_ok ? m : 0) * P.ld_bf16 + n0 + col0;
         const uint32_t tcol = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(buf * BN + col0);
         mbar_wait(&acc_full[buf], uint32_t((t >> 1) & 1));
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         __syncwarp();
         uint32_t va[16], vb[16], o[8];
         tmem_ld16_nowait(tcol, va);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld_wait();
         tmem_ld16_nowait(tcol + 16, vb);
-        ws2_act16(va, bs, act, o);
+        bias_act16(va, bs, act, o);
         if (row_ok) stg256(orow, o);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld_wait();
         tmem_ld16_nowait(tcol + 32, va);
-        ws2_act16(vb, bs + 16, act, o);
+        bias_act16(vb, bs + 16, act, o);
         if (row_ok) stg256(orow + 16, o);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld_wait();
         tmem_ld16_nowait(tcol + 48, vb);
-        ws2_act16(va, bs + 32, act, o);
+        bias_act16(va, bs + 32, act, o);
         if (row_ok) stg256(orow + 32, o);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tmem_ld_wait();
+        tc_fence_before();
         __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(buf ? leader_empty1 : leader_empty0) : "memory");
-        ws2_act16(vb, bs + 48, act, o);
+        if (lane == 0) mbar_arrive_cluster(buf ? leader_empty1 : leader_empty0);
+        bias_act16(vb, bs + 48, act, o);
         if (row_ok) stg256(orow + 48, o);
       }
     } else
@@ -460,49 +458,47 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1) tc_w
       const uint32_t tcol = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(buf * BN + col0);
       // the bulk store that last read this staging tile (ntiles row tiles ago) must have drained it
       if (lane == 0) {
-        if (ntiles == 1) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-        else asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        if (ntiles == 1) bulk_wait_read<0>();
+        else bulk_wait_read<1>();
       }
       mbar_wait(&acc_full[buf], uint32_t((t >> 1) & 1));
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       __syncwarp();
       uint32_t va[16], vb[16];
       tmem_ld16_nowait(tcol, va);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      tmem_ld_wait();
       tmem_ld16_nowait(tcol + 16, vb);
       ws2_finish16(va, bs, act, my_row, sw, 0);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      tmem_ld_wait();
       tmem_ld16_nowait(tcol + 32, va);
       ws2_finish16(vb, bs + 16, act, my_row, sw, 1);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      tmem_ld_wait();
       tmem_ld16_nowait(tcol + 48, vb);
       ws2_finish16(va, bs + 32, act, my_row, sw, 2);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      tmem_ld_wait();
       // every accumulator column of this warp has been read: release the TMEM buffer to the leader's MMA before the
       // last quarter of the math
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(buf ? leader_empty1 : leader_empty0) : "memory");
+      if (lane == 0) mbar_arrive_cluster(buf ? leader_empty1 : leader_empty0);
       ws2_finish16(vb, bs + 48, act, my_row, sw, 3);
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
         if (mq < P.M) {  // rows >= M and columns >= N inside the box are clipped by the tensor map
-          asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(tm_out)),
-                       "r"(sbase), "r"(n0 + col0), "r"(mq)
-                       : "memory");
+          tma_store_2d(tm_out, sbase, n0 + col0, mq);
         }
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        bulk_commit();
       }
     }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    if (lane == 0) bulk_wait<0>();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   cluster_sync_all();  // the peer may still be reading this CTA's operands / arriving on its barriers
   if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc<2, TMEM_COLS>(tmem_base);
   }
 }
 
