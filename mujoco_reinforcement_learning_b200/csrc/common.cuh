@@ -46,6 +46,57 @@ void count_launch();
     if (_r != B200PPO_OK) return _r; \
   } while (0)
 
+// Owns one cudaMalloc'd array and its capacity in elements; frees it when destroyed.  Never give one static storage
+// duration: its destructor would run after the CUDA runtime has shut down.
+template <typename T>
+class DevBuf {
+ public:
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  DevBuf(DevBuf&& o) noexcept : p_(o.p_), cap_(o.cap_) { o.p_ = nullptr; o.cap_ = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    std::swap(p_, o.p_);
+    std::swap(cap_, o.cap_);
+    return *this;
+  }
+  ~DevBuf() { reset(); }
+
+  // Frees what it holds (without synchronising), then allocates max(elems, 1) elements, zeroed on request.
+  int alloc(int64_t elems, bool zero = false) {
+    reset();
+    if (elems <= 0) elems = 1;
+    cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&p_), size_t(elems) * sizeof(T));
+    if (e != cudaSuccess) {
+      p_ = nullptr;
+      set_error("cudaMalloc(%lld bytes) failed: %s", (long long)(elems * sizeof(T)), cudaGetErrorString(e));
+      return e == cudaErrorMemoryAllocation ? B200PPO_ENOMEM : B200PPO_ECUDA;
+    }
+    cap_ = elems;
+    if (zero) B2_CUDA(cudaMemset(p_, 0, size_t(elems) * sizeof(T)));
+    return B200PPO_OK;
+  }
+  // Room for `elems` elements.  Growing waits for the device (queued work may still use the old array) and drops the
+  // contents; after a failure the buffer is empty, so the next call tries again.
+  int grow(int64_t elems) {
+    if (elems <= cap_) return B200PPO_OK;
+    B2_CUDA(cudaDeviceSynchronize());
+    return alloc(elems);
+  }
+  void reset() {
+    if (p_ != nullptr) cudaFree(p_);
+    p_ = nullptr;
+    cap_ = 0;
+  }
+  T* get() const { return p_; }
+  operator T*() const { return p_; }
+  int64_t cap() const { return cap_; }
+
+ private:
+  T* p_ = nullptr;
+  int64_t cap_ = 0;
+};
+
 inline int num_sms() {
   static int sms = 0;
   if (sms == 0) {

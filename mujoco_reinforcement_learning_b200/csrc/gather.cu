@@ -13,6 +13,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "gather.cuh"
 #include "tc_ptx.cuh"
 
 namespace b200ppo {
@@ -198,44 +199,42 @@ static inline unsigned gather_grid(int64_t count, int warps_per_block) {
   return unsigned(blocks < 1 ? 1 : blocks);
 }
 
-int launch_gather_chunked(const int64_t* idx, int64_t count, int64_t n_rows, int64_t chunk, int64_t chunk_stride,
-                          int64_t chunk_offset, const float* obs, int obs_dim, const float* act, int act_dim,
-                          const float* logp, const float* adv, const float* tgt, float* obs_o, float* act_o,
-                          float* logp_o, float* adv_o, float* tgt_o, int32_t* err_flag, cudaStream_t st) {
-  if (count == 0) return B200PPO_OK;
+int launch_gather_chunked(const GatherJob& j, const float* obs, int obs_dim, float* obs_o, cudaStream_t st) {
+  if (j.count == 0) return B200PPO_OK;
   const bool vec = (obs_dim % 4 == 0) && aligned16(obs) && aligned16(obs_o);
   const size_t tma_smem = size_t(32) * obs_dim * 4;
-  if (vec && tma_smem <= 56 * 1024 && count >= 4096) {  // bulk-copy engine path (rows are whole 16-byte multiples)
+  if (vec && tma_smem <= 56 * 1024 && j.count >= 4096) {  // bulk-copy engine path (rows are whole 16-byte multiples)
     static bool configured = false;
     if (!configured) {
       B2_CUDA(cudaFuncSetAttribute(gather_minibatch_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 56 * 1024));
       configured = true;
     }
     const int per_sm = int(std::max<size_t>(1, std::min<size_t>(16, (200 * 1024) / std::max<size_t>(tma_smem, 1))));
-    int64_t blocks = std::min<int64_t>((count + 31) / 32, int64_t(num_sms()) * per_sm);
-    gather_minibatch_tma_kernel<<<unsigned(blocks), 32, tma_smem, st>>>(idx, count, n_rows, chunk, chunk_stride, chunk_offset, obs,
-                                                                        obs_dim, act, act_dim, logp, adv, tgt, obs_o, act_o, logp_o,
-                                                                        adv_o, tgt_o, err_flag, ObsParts{});
+    int64_t blocks = std::min<int64_t>((j.count + 31) / 32, int64_t(num_sms()) * per_sm);
+    gather_minibatch_tma_kernel<<<unsigned(blocks), 32, tma_smem, st>>>(j.idx, j.count, j.n_rows, j.chunk, j.chunk_stride,
+                                                                        j.chunk_offset, obs, obs_dim, j.act, j.act_dim, j.logp,
+                                                                        j.adv, j.tgt, obs_o, j.act_o, j.logp_o, j.adv_o, j.tgt_o,
+                                                                        j.err_flag, ObsParts{});
     B2_LAUNCH_CHECK();
     return B200PPO_OK;
   }
-  dim3 block(256), grid(gather_grid(count, 8));
+  dim3 block(256), grid(gather_grid(j.count, 8));
   if (vec)
-    gather_minibatch_kernel<true><<<grid, block, 0, st>>>(idx, count, n_rows, chunk, chunk_stride, chunk_offset, obs, obs_dim, act, act_dim, logp, adv, tgt, obs_o, act_o, logp_o, adv_o, tgt_o, err_flag);
+    gather_minibatch_kernel<true><<<grid, block, 0, st>>>(j.idx, j.count, j.n_rows, j.chunk, j.chunk_stride, j.chunk_offset, obs,
+                                                          obs_dim, j.act, j.act_dim, j.logp, j.adv, j.tgt, obs_o, j.act_o,
+                                                          j.logp_o, j.adv_o, j.tgt_o, j.err_flag);
   else
-    gather_minibatch_kernel<false><<<grid, block, 0, st>>>(idx, count, n_rows, chunk, chunk_stride, chunk_offset, obs, obs_dim, act, act_dim, logp, adv, tgt, obs_o, act_o, logp_o, adv_o, tgt_o, err_flag);
+    gather_minibatch_kernel<false><<<grid, block, 0, st>>>(j.idx, j.count, j.n_rows, j.chunk, j.chunk_stride, j.chunk_offset, obs,
+                                                           obs_dim, j.act, j.act_dim, j.logp, j.adv, j.tgt, obs_o, j.act_o,
+                                                           j.logp_o, j.adv_o, j.tgt_o, j.err_flag);
   B2_LAUNCH_CHECK();
   return B200PPO_OK;
 }
 
-// Bulk-copy gather whose observation rows come from `n_parts` arrays of `rows_per_part` rows each (row_floats floats per
-// row, a multiple of 4, every array 16-byte aligned).
-int launch_gather_parts(const int64_t* idx, int64_t count, int64_t n_rows, int64_t chunk, int64_t chunk_stride, int64_t chunk_offset,
-                        const float* const* obs_parts, int n_parts, int64_t rows_per_part, int row_floats, const float* act,
-                        int act_dim, const float* logp, const float* adv, const float* tgt, float* obs_o, float* act_o,
-                        float* logp_o, float* adv_o, float* tgt_o, int32_t* err_flag, cudaStream_t st) {
-  if (count == 0) return B200PPO_OK;
-  B2_CHECK_ARG(n_parts >= 1 && n_parts <= 8 && rows_per_part > 0 && n_rows <= rows_per_part * n_parts, "gather: bad parts");
+int launch_gather_parts(const GatherJob& j, const float* const* obs_parts, int n_parts, int64_t rows_per_part, int row_floats,
+                        float* obs_o, cudaStream_t st) {
+  if (j.count == 0) return B200PPO_OK;
+  B2_CHECK_ARG(n_parts >= 1 && n_parts <= 8 && rows_per_part > 0 && j.n_rows <= rows_per_part * n_parts, "gather: bad parts");
   const size_t tma_smem = size_t(32) * row_floats * 4;
   B2_CHECK_ARG(row_floats % 4 == 0 && tma_smem <= 56 * 1024 && aligned16(obs_o), "gather from parts: rows must be 16-byte multiples <= 1792 bytes");
   ObsParts parts{};
@@ -251,24 +250,22 @@ int launch_gather_parts(const int64_t* idx, int64_t count, int64_t n_rows, int64
     configured = true;
   }
   const int per_sm = int(std::max<size_t>(1, std::min<size_t>(16, (200 * 1024) / std::max<size_t>(tma_smem, 1))));
-  int64_t blocks = std::min<int64_t>((count + 31) / 32, int64_t(num_sms()) * per_sm);
-  gather_minibatch_tma_kernel<<<unsigned(blocks), 32, tma_smem, st>>>(idx, count, n_rows, chunk, chunk_stride, chunk_offset, nullptr,
-                                                                      row_floats, act, act_dim, logp, adv, tgt, obs_o, act_o, logp_o,
-                                                                      adv_o, tgt_o, err_flag, parts);
+  int64_t blocks = std::min<int64_t>((j.count + 31) / 32, int64_t(num_sms()) * per_sm);
+  gather_minibatch_tma_kernel<<<unsigned(blocks), 32, tma_smem, st>>>(j.idx, j.count, j.n_rows, j.chunk, j.chunk_stride,
+                                                                      j.chunk_offset, nullptr, row_floats, j.act, j.act_dim, j.logp,
+                                                                      j.adv, j.tgt, obs_o, j.act_o, j.logp_o, j.adv_o, j.tgt_o,
+                                                                      j.err_flag, parts);
   B2_LAUNCH_CHECK();
   return B200PPO_OK;
 }
 
-int launch_gather_chunked_bf16(const int64_t* idx, int64_t count, int64_t n_rows, int64_t chunk, int64_t chunk_stride,
-                               int64_t chunk_offset, const float* obs, int obs_dim, const float* act, int act_dim,
-                               const float* logp, const float* adv, const float* tgt, __nv_bfloat16* obs_o, int pitch,
-                               float* act_o, float* logp_o, float* adv_o, float* tgt_o, int32_t* err_flag, cudaStream_t st) {
-  if (count == 0) return B200PPO_OK;
+int launch_gather_chunked_bf16(const GatherJob& j, const float* obs, int obs_dim, __nv_bfloat16* obs_o, int pitch, cudaStream_t st) {
+  if (j.count == 0) return B200PPO_OK;
   const int vec = (obs_dim % 4 == 0) && aligned16(obs) && (pitch % 4 == 0) && ((uintptr_t)obs_o % 8 == 0);
-  dim3 block(256), grid(gather_grid(count, 8));
-  gather_minibatch_bf16_kernel<<<grid, block, 0, st>>>(idx, count, n_rows, chunk, chunk_stride, chunk_offset, obs, obs_dim,
-                                                       act, act_dim, logp, adv, tgt, obs_o, pitch, act_o, logp_o, adv_o,
-                                                       tgt_o, err_flag, vec);
+  dim3 block(256), grid(gather_grid(j.count, 8));
+  gather_minibatch_bf16_kernel<<<grid, block, 0, st>>>(j.idx, j.count, j.n_rows, j.chunk, j.chunk_stride, j.chunk_offset, obs,
+                                                       obs_dim, j.act, j.act_dim, j.logp, j.adv, j.tgt, obs_o, pitch, j.act_o,
+                                                       j.logp_o, j.adv_o, j.tgt_o, j.err_flag, vec);
   B2_LAUNCH_CHECK();
   return B200PPO_OK;
 }
@@ -287,9 +284,11 @@ extern "C" B2_EXPORT int b200ppo_gather_minibatch(const int64_t* idx, int64_t co
                "b200ppo_gather_minibatch: missing output for a supplied leaf");
   B2_CHECK_ARG(count >= 0 && n_rows >= 0 && obs_dim > 0 && obs_dim < (1 << 30) && act_dim >= 0 && act_dim < (1 << 30),
                "b200ppo_gather_minibatch: bad sizes");
-  return launch_gather_chunked(idx, count, n_rows, count, count, 0, obs, int(obs_dim), action, int(act_dim), logp,
-                               advantage, target, obs_out, action_out, logp_out, advantage_out, target_out, err_flag,
-                               static_cast<cudaStream_t>(stream));
+  GatherJob j{};
+  j.idx = idx; j.count = count; j.n_rows = n_rows; j.chunk = count; j.chunk_stride = count; j.chunk_offset = 0;
+  j.act = action; j.act_dim = int(act_dim); j.logp = logp; j.adv = advantage; j.tgt = target;
+  j.act_o = action_out; j.logp_o = logp_out; j.adv_o = advantage_out; j.tgt_o = target_out; j.err_flag = err_flag;
+  return launch_gather_chunked(j, obs, int(obs_dim), obs_out, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" B2_EXPORT int b200ppo_gather_rows(const void* src, int64_t row_bytes, int64_t n_rows, const int64_t* idx,

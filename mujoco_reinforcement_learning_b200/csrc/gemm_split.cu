@@ -34,32 +34,8 @@ static inline int pad64(int x) { return (x + 63) / 64 * 64; }
 int64_t split_arena_elems(int64_t rows, int cols) { return (rows * 3 * pad64(cols + 1) + 511) / 512 * 512; }
 
 int split_arena_reserve(SplitArena& a, int64_t elems) {
-  if (elems <= a.cap) return B200PPO_OK;
-  B2_CUDA(cudaDeviceSynchronize());
-  if (a.base != nullptr) cudaFree(a.base);
-  a.base = nullptr;
-  a.cap = 0;
-  split_arena_reset(a);
-  if (a.amax == nullptr && cudaMalloc(reinterpret_cast<void**>(&a.amax), SplitArena::kMaxEntries * sizeof(float)) != cudaSuccess) {
-    set_error("cudaMalloc of the operand-scale array failed");
-    return B200PPO_ENOMEM;
-  }
-  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&a.base), size_t(elems) * sizeof(__nv_bfloat16));
-  if (e != cudaSuccess) {
-    set_error("cudaMalloc(%lld bytes) for the three-term operand arena failed: %s", (long long)(elems * 2), cudaGetErrorString(e));
-    return e == cudaErrorMemoryAllocation ? B200PPO_ENOMEM : B200PPO_ECUDA;
-  }
-  a.cap = elems;
-  return B200PPO_OK;
-}
-
-void split_arena_free(SplitArena& a) {
-  if (a.base != nullptr) cudaFree(a.base);
-  if (a.amax != nullptr) cudaFree(a.amax);
-  a.base = nullptr;
-  a.amax = nullptr;
-  a.cap = a.used = 0;
-  a.n = 0;
+  if (a.amax == nullptr) B2_TRY(a.amax.alloc(SplitArena::kMaxEntries));
+  return a.base.grow(elems);
 }
 
 // ---- the split pass ------------------------------------------------------------------------------------------------------
@@ -279,9 +255,9 @@ static int get_split(SplitArena& arena, SplitJobs& jobs, const float* src, int64
   }
   const int cp = pad64(cols + 1);
   const int64_t elems = split_arena_elems(rows, cols);
-  if (arena.n >= SplitArena::kMaxEntries || arena.used + elems > arena.cap || jobs.n >= kMaxSplitJobs) {
+  if (arena.n >= SplitArena::kMaxEntries || arena.used + elems > arena.base.cap() || jobs.n >= kMaxSplitJobs) {
     set_error("three-term operand arena exhausted (%d entries, %lld of %lld elements used, %lld more asked)", arena.n,
-              (long long)arena.used, (long long)arena.cap, (long long)elems);
+              (long long)arena.used, (long long)arena.base.cap(), (long long)elems);
     return B200PPO_EINVAL;
   }
   __nv_bfloat16* dst = arena.base + arena.used;
@@ -394,7 +370,7 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
       const int ones = (p.epilogue == EPI_BIAS_TANH || p.epilogue == EPI_BIAS_RELU) ? 1 : 0;
       bool known = false;
       for (int e = 0; e < arena.n; ++e) known |= arena.e[e].src == p.C && arena.e[e].rows == p.M && arena.e[e].cols == p.N;
-      if (!known && arena.used + oelems <= arena.cap) {
+      if (!known && arena.used + oelems <= arena.base.cap()) {
         __nv_bfloat16* odst = arena.base + arena.used;
         arena.used += oelems;
         arena.e[arena.n++] = SplitArena::Entry{p.C, int64_t(p.M), int64_t(p.ldc), p.N, ones, ocp, 3, odst, arena.amax};
@@ -431,10 +407,9 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
   // debug: B200PPO_SPLIT_TRACE=<n> prints phase marks (cycles) of every 37th CTA of the n-th launch
   static const char* trace_env = getenv("B200PPO_SPLIT_TRACE");
   static int calls = 0;
-  long long* trace = nullptr;
+  DevBuf<long long> trace;  // declared before `dump`, so freed after it has printed
   if (trace_env != nullptr && ++calls == atoi(trace_env)) {
-    B2_CUDA(cudaMalloc(&trace, 64 * 8 * sizeof(long long)));
-    B2_CUDA(cudaMemset(trace, 0, 64 * 8 * sizeof(long long)));
+    B2_TRY(trace.alloc(64 * 8, true));
     tg.trace = trace;
   }
   struct TraceDump {
@@ -444,7 +419,6 @@ int launch_gemm_group_split(const GemmGroup& g, SplitArena& arena, cudaStream_t 
       cudaStreamSynchronize(st);
       long long h[64 * 8];
       cudaMemcpy(h, t, sizeof(h), cudaMemcpyDeviceToHost);
-      cudaFree(t);
       if (persistent) {  // tc_persist_kernel: the tiles of CTA 0 (slot 3 = epilogue enters, before it waits for the accumulator)
         const long long t0 = h[5];
         fprintf(stderr, "persistent split GEMM, %d tiles, CTA 0: tile | producer first, last load | issuer: accumulator, first operands, last MMA | epilogue: enters, done\n", tiles);
@@ -494,16 +468,6 @@ int launch_absmax(const float* src, int64_t rows, int cols, int64_t ld, float* o
 }  // namespace b200ppo
 
 // ---- test hook --------------------------------------------------------------------------------------------------------------
-namespace b200ppo {
-__global__ void sum_partials_kernel(const float* __restrict__ part, int splits, int64_t stride, int64_t n, float* __restrict__ out) {
-  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  float s = 0.f;
-  for (int k = 0; k < splits; ++k) s += part[k * stride + i];
-  out[i] = s;
-}
-}  // namespace b200ppo
-
 using namespace b200ppo;
 
 extern "C" B2_EXPORT int b200ppo_debug_gemm_split(const float* A, const float* B, float* C, float* bias_grad, int32_t M, int32_t N,
@@ -518,8 +482,8 @@ extern "C" B2_EXPORT int b200ppo_debug_gemm_split(const float* A, const float* B
                        4 * (int64_t(M) + K + 2048);
   B2_TRY(split_arena_reserve(arena, need));
   const int64_t mn = int64_t(M) * N, stride = (mn + M + 3) / 4 * 4;
-  float* part = nullptr;
-  B2_CUDA(cudaMalloc(&part, size_t(split_k) * stride * 4));
+  DevBuf<float> part;
+  B2_TRY(part.alloc(int64_t(split_k) * stride));
   GemmGroup g{};
   GemmProblem p{};
   p.A = A; p.B = B; p.C = part; p.ldc = N;
@@ -532,16 +496,14 @@ extern "C" B2_EXPORT int b200ppo_debug_gemm_split(const float* A, const float* B
   gemm_group_add(g, p, 64, 64, split_k);
   int rc = launch_gemm_group_split(g, arena, st);
   if (rc == B200PPO_OK) {
-    sum_partials_kernel<<<unsigned((mn + 255) / 256), 256, 0, st>>>(part, split_k, stride, mn, C);
+    sum_splits_kernel<<<unsigned((mn + 255) / 256), 256, 0, st>>>(part, split_k, stride, mn, C);
     count_launch();
     if (bias_grad != nullptr) {
-      sum_partials_kernel<<<unsigned((M + 255) / 256), 256, 0, st>>>(part + mn, split_k, stride, M, bias_grad);
+      sum_splits_kernel<<<unsigned((M + 255) / 256), 256, 0, st>>>(part + mn, split_k, stride, M, bias_grad);
       count_launch();
     }
   }
   cudaStreamSynchronize(st);
-  cudaFree(part);
-  split_arena_free(arena);
   if (rc != B200PPO_OK) return rc;
   B2_CUDA(cudaGetLastError());
   return B200PPO_OK;

@@ -17,10 +17,10 @@ struct SplitArena {
     float* amax;  // two-term mode: the largest magnitude of src, the source of its scale
   };
   static constexpr int kMaxEntries = 96;  // 2 nets x B200PPO_MAX_LAYERS x (activation, two dL/dz views, weights) and room to spare
-  __nv_bfloat16* base = nullptr;
-  float* amax = nullptr;      // [kMaxEntries] largest magnitude of every entry's source (two-term mode: the scale comes from it)
+  DevBuf<__nv_bfloat16> base;
+  DevBuf<float> amax;         // [kMaxEntries] largest magnitude of every entry's source (two-term mode: the scale comes from it)
   bool amax_zeroed = false;   // since the last reset
-  int64_t cap = 0, used = 0;  // elements
+  int64_t used = 0;           // elements of base
   Entry e[kMaxEntries];
   int n = 0;
   // 3: three bf16 terms per value, six products — 24-bit operands, the 1e-5 variant (default).  2: two fp16 terms of the
@@ -29,10 +29,9 @@ struct SplitArena {
   int terms = 3;
 };
 
-int split_arena_reserve(SplitArena& a, int64_t elems);  // (re)allocates; synchronises the device when it has to grow
+int split_arena_reserve(SplitArena& a, int64_t elems);  // grows base to `elems` (DevBuf::grow)
 inline void split_arena_reset(SplitArena& a) { a.used = 0; a.n = 0; a.amax_zeroed = false; }
-void split_arena_free(SplitArena& a);
-// samples one tensor-core accumulator of a weight gradient may sum (see backward_nets in api.cu)
+// samples one tensor-core accumulator of a weight gradient may sum (see backward_nets in passes.cu)
 constexpr int kSplitChain = 512;
 // elements one [rows][cols] operand occupies in the arena
 int64_t split_arena_elems(int64_t rows, int cols);

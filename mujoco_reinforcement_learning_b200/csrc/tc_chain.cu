@@ -808,9 +808,8 @@ int launch_tc_chain(const ChainArgs& a, cudaStream_t st, int* grid_out, bool inf
   static const char* trace_env = getenv("B200PPO_CHAIN_TRACE");
   static int calls = 0;
   if (trace_env != nullptr && !infer && ++calls == atoi(trace_env)) {
-    long long* tr = nullptr;
-    B2_CUDA(cudaMalloc(&tr, (60 * 8 + 64 * 4) * sizeof(long long)));
-    B2_CUDA(cudaMemset(tr, 0, (60 * 8 + 64 * 4) * sizeof(long long)));
+    DevBuf<long long> tr;
+    B2_TRY(tr.alloc(60 * 8 + 64 * 4, true));
     ChainArgs b = a;
     b.trace = tr;
     B2_CUDA(launch_pdl(kernel, dim3(2 * pairs), dim3(CH_THREADS), CH_SMEM, st, b));
@@ -818,7 +817,6 @@ int launch_tc_chain(const ChainArgs& a, cudaStream_t st, int* grid_out, bool inf
     B2_CUDA(cudaStreamSynchronize(st));
     long long h[60 * 8 + 64 * 4];
     B2_CUDA(cudaMemcpy(h, tr, sizeof(h), cudaMemcpyDeviceToHost));
-    cudaFree(tr);
     static const char* names[10] = {"L1a", "L1c", "L2a", "L2c", "L3a", "L3c", "D3c", "D3a", "D2c", "D2a"};
     fprintf(stderr, "chain kernel, pair 0 (M = %d, %d pairs): step | operands ready, issued | accumulator seen, epilogue done\n", a.M, pairs);
     for (int g = 0; g < 60 && h[g * 8] != 0; ++g)

@@ -296,13 +296,13 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
   const int64_t a_rows = a_mn_major ? K : M, a_cols = a_mn_major ? M : K;
   const int64_t b_rows = b_mn_major ? K : N, b_cols = b_mn_major ? N : K;
   const int64_t a_pitch = pad8(a_cols), b_pitch = pad8(b_cols);
-  __nv_bfloat16 *Ab = nullptr, *Bb = nullptr;
-  float* part = nullptr;
+  DevBuf<__nv_bfloat16> Ab, Bb, out_bf16, auxb;
+  DevBuf<float> part;
   if (split_k < 1) split_k = 1;
-  B2_CUDA(cudaMalloc(&Ab, a_rows * a_pitch * 2));
-  B2_CUDA(cudaMalloc(&Bb, b_rows * b_pitch * 2));
+  B2_TRY(Ab.alloc(a_rows * a_pitch));
+  B2_TRY(Bb.alloc(b_rows * b_pitch));
   const int64_t mn = int64_t(M) * N, stride = (mn + 3) / 4 * 4;
-  B2_CUDA(cudaMalloc(&part, size_t(split_k) * stride * 4));
+  B2_TRY(part.alloc(int64_t(split_k) * stride));
   cast_pad_bf16_kernel<<<unsigned((a_rows * a_pitch + 255) / 256), 256, 0, st>>>(A, a_rows, a_cols, a_pitch, Ab);
   B2_LAUNCH_CHECK();
   cast_pad_bf16_kernel<<<unsigned((b_rows * b_pitch + 255) / 256), 256, 0, st>>>(B, b_rows, b_cols, b_pitch, Bb);
@@ -322,9 +322,9 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
     p.epilogue = TC_EPI_DGRAD; p.act = B200PPO_ACT_TANH;
     p.out_f32 = nullptr;
     const int64_t ld = (N + 7) / 8 * 8;
-    __nv_bfloat16* auxb = nullptr;
-    B2_CUDA(cudaMalloc(&p.out_bf16, size_t(M) * ld * 2));
-    B2_CUDA(cudaMalloc(&auxb, size_t(M) * ld * 2));
+    B2_TRY(out_bf16.alloc(M * ld));
+    B2_TRY(auxb.alloc(M * ld));
+    p.out_bf16 = out_bf16;
     cast_pad_bf16_kernel<<<unsigned((int64_t(M) * ld + 255) / 256), 256, 0, st>>>(C, M, N, ld, auxb);
     B2_LAUNCH_CHECK();
     p.ld_bf16 = int(ld); p.aux = auxb; p.ld_aux = int(ld);
@@ -332,7 +332,8 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
   if (bn == -3) {
     p.epilogue = TC_EPI_FWD; p.act = B200PPO_ACT_TANH;  // the production forward epilogue, bf16 output
     p.out_f32 = nullptr;
-    B2_CUDA(cudaMalloc(&p.out_bf16, size_t(M) * ((N + 7) / 8 * 8) * 2));
+    B2_TRY(out_bf16.alloc(int64_t(M) * ((N + 7) / 8 * 8)));
+    p.out_bf16 = out_bf16;
     p.ld_bf16 = (N + 7) / 8 * 8;
   }
   if (ws) bn = tc_ws_bn(N, K);
@@ -346,12 +347,9 @@ extern "C" B2_EXPORT int b200ppo_debug_tc_gemm(const float* A, const float* B, f
     count_launch();
   }
   cudaStreamSynchronize(st);
-  if (p.out_bf16 != nullptr) cudaFree(p.out_bf16);
-  if (p.aux != nullptr) cudaFree(const_cast<__nv_bfloat16*>(p.aux));
-  cudaFree(Ab); cudaFree(Bb); cudaFree(part);
   {
     std::lock_guard<std::mutex> lock(g_map_mutex);
-    g_map_cache.clear();  // the temporaries above are gone
+    g_map_cache.clear();  // the temporaries above are freed on return
   }
   if (rc != B200PPO_OK) return rc;
   B2_CUDA(cudaGetLastError());

@@ -143,4 +143,9 @@ int launch_tc_ws(const TcGroup& g, cudaStream_t st, int* grid_out = nullptr, boo
 // layer's input width without a ones-column, the bias gradient comes from a second MMA against a tile of ones.
 int launch_tc_wgrad2(const TcGroup& g, int max_split, cudaStream_t st, int* split_out);
 
+// debug helpers (tc_gemm.cu): out[i] = sum over the splits of part[k * stride + i]; bf16 rows [rows][pitch] -> dense fp32
+__global__ void sum_splits_kernel(const float* __restrict__ part, int splits, int64_t stride, int64_t n, float* __restrict__ out);
+__global__ void bf16_rows_to_f32_kernel(const __nv_bfloat16* __restrict__ src, int64_t rows, int64_t cols, int64_t pitch,
+                                        float* __restrict__ dst);
+
 }  // namespace b200ppo
