@@ -82,18 +82,13 @@ struct CastTable {
   int count;
 };
 
-// Block-level finish of the fused-epilogue loss partials: s_lc[0] = sum surrogate, [1] = sum huber, [2+j] = logstd grads.
+// Block-level finish of the fused-epilogue loss partials: the two losses, and the logstd gradient into s_lc[2 + j].
 __device__ __forceinline__ void combine_losses(const LossCombine& lc, float* s_lc, float* s_scr) {
   const int tid = threadIdx.x;
   const float s = combine_partials<256>(lc.partials, unsigned(lc.n_cta), 2 + lc.act_dim, tid, s_scr);
-  if (tid < 2 + lc.act_dim) s_lc[tid] = tid < 2 ? s : s - lc.ent_coef * lc.rank_share / float(lc.act_dim);
-  if (tid == 0 && lc.losses_out != nullptr) {
-    float ent = 0.f;  // mean over [B, A] of 0.5 + 0.5 log(2 pi) + log sigma_j
-    for (int j = 0; j < lc.act_dim; ++j) ent += 0.5f + 0.91893853320467274178f + logf(expf(lc.logstd[j]));
-    ent /= float(lc.act_dim);
-    lc.losses_out[0] = -s * lc.inv_global_batch - lc.ent_coef * ent * lc.rank_share;
-  }
-  if (tid == 1 && lc.losses_out != nullptr) lc.losses_out[1] = s * lc.inv_global_batch;
+  if (tid < 2 + lc.act_dim)
+    ppo_finish_column(lc, lc.ent_coef, lc.rank_share, tid, s, [&](int j) { return logf(expf(lc.logstd[j])); }, lc.losses_out,
+                      s_lc + 2, nullptr);
   __syncthreads();
 }
 

@@ -2,6 +2,7 @@
 #pragma once
 #include "cast.cuh"
 #include "common.cuh"
+#include "ppo_math.cuh"
 
 namespace b200ppo {
 
@@ -21,12 +22,12 @@ int launch_adam(float* params, const float* grads, int n_partials, int64_t parti
 
 // When the loss sums come out of the fused PPO epilogues as per-CTA partials (tc_common.cuh), the kernel that consumes
 // the gradients also finishes them: fixed-order sum over the CTAs, the two loss values, and d loss / d logstd.
-struct LossCombine {
-  const float* partials = nullptr;  // [n_cta][2 + act_dim]; nullptr = nothing to combine
-  int n_cta = 0, act_dim = 0;
+// The operands used: partials ([n_cta][2 + act_dim]; nullptr = nothing to combine), act_dim, logstd (current actor_logstd,
+// for the entropy term) and inv_global_batch.
+struct LossCombine : PpoOperands {
+  int n_cta = 0;
   int64_t logstd_off = 0;           // element offset of actor_logstd in the flat buffers
-  const float* logstd = nullptr;    // current actor_logstd (for the entropy term)
-  float inv_global_batch = 0.f, ent_coef = 0.f, rank_share = 1.f;
+  float ent_coef = 0.f, rank_share = 1.f;
   float* losses_out = nullptr;      // [2]
 };
 

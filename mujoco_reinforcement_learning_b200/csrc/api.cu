@@ -164,12 +164,9 @@ extern "C" B2_EXPORT int b200ppo_evaluate(b200ppo_ctx* ctx, const float* params,
   float* acts[2] = {ctx->ws_act[0], ctx->ws_act[1]};
   float* outs[2] = {ctx->ws_out[0], value ? value : ctx->ws_out[1]};
   B2_TRY(forward_nets(ctx, params, obs, batch, 3, acts, outs, st, false, fresh_arena(ctx)));
-  LossArgs la{};
-  la.mean = outs[0]; la.logstd = params + ctx->logstd_off; la.action = action; la.batch = batch;
-  la.act_dim = ctx->net[0].out_dim(); la.final_tanh = ctx->net[0].d.final_tanh; la.out_scale = ctx->net[0].d.out_scale;
-  la.inv_global_batch = 1.f / float(batch); la.rank_share = 1.f;
-  la.logp_out = logp; la.entropy_out = entropy;
-  la.partials = ctx->loss_partials; la.ticket = ctx->ticket;
+  LossArgs la{ppo_operands(ctx, params, nullptr, batch, action, nullptr, nullptr, nullptr)};
+  la.mean = outs[0]; la.batch = batch; la.out_scale = ctx->net[0].d.out_scale; la.rank_share = 1.f;
+  la.logp_out = logp; la.entropy_out = entropy; la.ticket = ctx->ticket;
   return launch_ppo_loss(la, st);
 }
 

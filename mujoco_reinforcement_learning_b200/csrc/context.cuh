@@ -182,6 +182,9 @@ int launch_chain(b200ppo_ctx* ctx, const float* params, const __nv_bfloat16* xb,
 int minibatch_fwd_bwd(b200ppo_ctx* ctx, const float* params, const float* obs, const __nv_bfloat16* obs_b, const float* action,
                       const float* old_logp, const float* adv, const float* tgt, int64_t B, const b200ppo_hparams* hp,
                       float* losses_dev, int* split_out, int* loss_ctas_out, cudaStream_t st);
+// the per-row loss operands of a B-row minibatch (hp may be null when no loss is computed)
+PpoOperands ppo_operands(const b200ppo_ctx* ctx, const float* params, const b200ppo_hparams* hp, int64_t B, const float* action,
+                         const float* old_logp, const float* adv, const float* tgt);
 LossCombine make_loss_combine(const b200ppo_ctx* ctx, const float* params, int loss_ctas, int64_t B, const b200ppo_hparams* hp,
                               float* losses_out);
 

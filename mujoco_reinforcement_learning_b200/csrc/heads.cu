@@ -4,20 +4,19 @@
 //   * the last Linear of the actor (+ output_max_value * tanh) and of the critic
 //     (src/models/linear/actor.py:25-30, src/models/critic.py:22-25),
 //   * Normal.log_prob(...).sum(1), entropy, ratio / clamp / min surrogate and Huber loss with their autograd
-//     seeds (src/entities/algorithms/ppo.py:113-132; formulas in SURVEY.md §8a row a10),
+//     seeds (src/entities/algorithms/ppo.py:113-132; the math: ppo_math.cuh),
 //   * the dgrad of those last Linears through the hidden activation: dZ_hidden = (dZ_out W_out) * act'(H).
 // The output layers are tall-skinny (N = act_dim <= 32 and N = 1): GEMV-shaped work that would leave a GEMM tile
 // ~90% empty, so a warp owns a sample row instead: lanes split the hidden dimension (coalesced 128-bit loads of
 // the row), W_out lives in shared memory, the act_dim dot products are butterfly-reduced, the loss terms are
-// computed on lanes [0, act_dim) and dZ_hidden is written back row-coalesced (fp32 and/or bf16 for the
-// tensor-core path).  Loss sums and the logstd gradient are reduced in a fixed order (deterministic).
+// computed on lanes [0, act_dim) and dZ_hidden is written back row-coalesced.  Loss sums and the logstd gradient are
+// reduced in a fixed order (deterministic).
 #include <algorithm>
 
 #include "heads.cuh"
 
 namespace b200ppo {
 
-constexpr float kLogSqrt2Pi = 0.91893853320467274178f;
 constexpr int kHeadsWarps = 8;
 constexpr int kHeadsThreads = kHeadsWarps * 32;
 constexpr int kMaxChunk = 8;  // hidden width <= 32 lanes * 4 floats * kMaxChunk = 1024 (kernel is templated on the
@@ -32,7 +31,6 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
   float* s_w3a = smem;                 // [A][Ha]
   float* s_w3c = s_w3a + A * Ha;       // [Hc]
   float* s_red = s_w3c + Hc;           // [kHeadsWarps][2 + 32], reused (>= kHeadsThreads floats) by the final combine
-  __shared__ bool s_last;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   {  // weights -> smem: 128-bit loads, unrolled so the L2 round trips overlap instead of serialising on the store
     const int n4 = (A * Ha) >> 2;
@@ -48,13 +46,11 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
   const bool jl = lane < A;
   float logsig = 0.f, inv_var = 0.f, two_var = 1.f, b3a = 0.f;
   if (jl) {
-    const float sig = expf(__ldg(a.logstd + lane));
-    const float var = sig * sig;
-    logsig = logf(sig); inv_var = 1.f / var; two_var = 2.f * var;
+    const PpoSigma c = ppo_sigma(__ldg(a.logstd + lane));
+    logsig = c.logsig; inv_var = c.inv_var; two_var = c.two_var;
     b3a = __ldg(a.b3a + lane);
   }
   const float b3c = __ldg(a.b3c);
-  const float lo = 1.f - a.clip_eps, hi = 1.f + a.clip_eps;
   const int nca = (Ha + 127) / 128, ncc = (Hc + 127) / 128;
 
   float acc_surr = 0.f, acc_hub = 0.f, acc_dl = 0.f;  // acc_dl: lane j accumulates d loss / d logstd_j
@@ -96,25 +92,16 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
       const float z = zmine + b3a;
       if (a.final_tanh) { th = tanhf(z); mean = a.out_scale * th; } else { mean = z; }
       d = act_in - mean;
-      lp_term = -(d * d) / two_var - logsig - kLogSqrt2Pi;
-      if (a.mean_out != nullptr) a.mean_out[b * A + lane] = mean;
+      lp_term = ppo_logp_term(d, logsig, two_var);
     }
-    const float lp = warp_sum(lp_term);
-    const float ratio = expf(lp - old_lp);
-    const float s1 = ratio * adv, s2 = fminf(fmaxf(ratio, lo), hi) * adv;
-    const float w1 = s1 < s2 ? 1.f : (s1 > s2 ? 0.f : 0.5f);
-    const float in_range = (ratio >= lo && ratio <= hi) ? 1.f : 0.f;
-    const float g_lp = -(w1 * adv + (1.f - w1) * adv * in_range) * a.inv_global_batch * ratio;
+    const PpoSurrogate ps = ppo_surrogate(warp_sum(lp_term), old_lp, adv, a.clip_eps, a.inv_global_batch);
     float dz3 = 0.f;
     if (jl) {
-      const float dn = d * inv_var;
-      dz3 = g_lp * dn;
-      if (a.final_tanh) dz3 *= a.out_scale * (1.f - th * th);
-      acc_dl += g_lp * (d * dn - 1.f);
+      dz3 = ppo_mean_seed(ps.g_lp, d, inv_var, a.final_tanh, a.out_scale, [&] { return th; });
+      acc_dl += ppo_logstd_term(ps.g_lp, d, inv_var);
       if (a.dz3_f32 != nullptr) a.dz3_f32[b * A + lane] = dz3;
     }
-    if (a.dz3_bf16 != nullptr && lane < a.dz3_pitch) a.dz3_bf16[b * a.dz3_pitch + lane] = __float2bfloat16_rn(dz3);
-    if (lane == 0) acc_surr += fminf(s1, s2);
+    if (lane == 0) acc_surr += ps.surr;
     // ---- actor dgrad through the hidden activation: dZ2a[k] = (sum_j dz3_j W3a[j,k]) * act'(h_k) --------------
     float4 g[NCHUNK];
 #pragma unroll
@@ -138,12 +125,6 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
         o.x = g[c].x * act_deriv(h[c].x, a.act); o.y = g[c].y * act_deriv(h[c].y, a.act);
         o.z = g[c].z * act_deriv(h[c].z, a.act); o.w = g[c].w * act_deriv(h[c].w, a.act);
         if (a.dz_a_f32 != nullptr) *reinterpret_cast<float4*>(a.dz_a_f32 + b * Ha + k) = o;
-        if (a.dz_a_bf16 != nullptr) {
-          const __nv_bfloat162 p0 = __floats2bfloat162_rn(o.x, o.y), p1 = __floats2bfloat162_rn(o.z, o.w);
-          uint2 w;
-          w.x = *reinterpret_cast<const uint32_t*>(&p0); w.y = *reinterpret_cast<const uint32_t*>(&p1);
-          *reinterpret_cast<uint2*>(a.dz_a_bf16 + b * a.dz_a_pitch + k) = w;
-        }
       }
     }
     // ---- critic: v = h_c . w3c + b3c ; Huber ; dZ2c -----------------------------------------------------------
@@ -157,16 +138,12 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
         pv = fmaf(h[c].x, w.x, pv); pv = fmaf(h[c].y, w.y, pv); pv = fmaf(h[c].z, w.z, pv); pv = fmaf(h[c].w, w.w, pv);
       }
     }
-    const float v = warp_sum(pv) + b3c;
-    const float e = v - target;
-    const float ae = fabsf(e);
-    const float dv = fminf(fmaxf(e, -1.f), 1.f) * a.inv_global_batch;
+    const PpoHuber hub = ppo_huber(warp_sum(pv) + b3c, target, a.inv_global_batch);
+    const float dv = hub.dv;
     if (lane == 0) {
-      acc_hub += ae < 1.f ? 0.5f * e * e : ae - 0.5f;
-      if (a.value_out != nullptr) a.value_out[b] = v;
+      acc_hub += hub.loss;
       if (a.dv_f32 != nullptr) a.dv_f32[b] = dv;
     }
-    if (a.dv_bf16 != nullptr && lane < a.dv_pitch) a.dv_bf16[b * a.dv_pitch + lane] = __float2bfloat16_rn(lane == 0 ? dv : 0.f);
 #pragma unroll
     for (int c = 0; c < NCHUNK; ++c) {
       const int k = c * 128 + lane * 4;
@@ -176,12 +153,6 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
         o.x = dv * w.x * act_deriv(h[c].x, a.act_c); o.y = dv * w.y * act_deriv(h[c].y, a.act_c);
         o.z = dv * w.z * act_deriv(h[c].z, a.act_c); o.w = dv * w.w * act_deriv(h[c].w, a.act_c);
         if (a.dz_c_f32 != nullptr) *reinterpret_cast<float4*>(a.dz_c_f32 + b * Hc + k) = o;
-        if (a.dz_c_bf16 != nullptr) {
-          const __nv_bfloat162 p0 = __floats2bfloat162_rn(o.x, o.y), p1 = __floats2bfloat162_rn(o.z, o.w);
-          uint2 w2;
-          w2.x = *reinterpret_cast<const uint32_t*>(&p0); w2.y = *reinterpret_cast<const uint32_t*>(&p1);
-          *reinterpret_cast<uint2*>(a.dz_c_bf16 + b * a.dz_c_pitch + k) = w2;
-        }
       }
     }
   }
@@ -197,28 +168,8 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_fused_kernel(const __grid
     for (int w = 0; w < kHeadsWarps; ++w) s += s_red[w * 34 + c];
     part[c] = s;
   }
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) s_last = (atomicAdd(a.ticket, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  {
-    const float s = combine_partials<kHeadsThreads>(a.partials, gridDim.x, 2 + A, tid, s_red);
-    const int c = tid;
-    if (c >= 2 + A) return;
-    if (c == 0) {
-      float ent = 0.f;
-      for (int j = 0; j < A; ++j) ent += 0.5f + kLogSqrt2Pi + logf(expf(__ldg(a.logstd + j)));
-      ent /= float(A);
-      if (a.losses != nullptr) a.losses[0] = -s * a.inv_global_batch - a.ent_coef * ent * a.rank_share;
-    } else if (c == 1) {
-      if (a.losses != nullptr) a.losses[1] = s * a.inv_global_batch;
-    } else if (a.logstd_grad != nullptr) {
-      a.logstd_grad[c - 2] = s - a.ent_coef * a.rank_share / float(A);
-    }
-    if (tid == 0) *a.ticket = 0u;
-  }
+  ppo_last_cta_finish<kHeadsThreads>(a, a.ent_coef, a.rank_share, a.ticket, s_red,
+                                     [&](int j) { return logf(expf(__ldg(a.logstd + j))); }, a.losses, a.logstd_grad, nullptr);
 }
 
 bool heads_supported(int act_dim, int hid_a, int hid_c) {

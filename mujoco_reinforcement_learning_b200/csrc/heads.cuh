@@ -1,37 +1,24 @@
 // Internal interface of the fused output-layer / loss / first-dgrad kernel (heads.cu).
 #pragma once
-#include <cuda_bf16.h>
-
-#include "common.cuh"
+#include "ppo_math.cuh"
 
 namespace b200ppo {
 
-struct HeadsArgs {
+struct HeadsArgs : PpoOperands {
   // inputs
   const float* h_a;  // [B, hid_a] last hidden activation of the actor (fp32)
   const float* h_c;  // [B, hid_c] last hidden activation of the critic
-  const float *w3a, *b3a, *w3c, *b3c, *logstd;
-  const float *action, *old_logp, *advantage, *target;
+  const float *w3a, *b3a, *w3c, *b3c;
   int64_t batch;
-  int act_dim, hid_a, hid_c;
+  int hid_a, hid_c;
   int act, act_c;  // hidden activation codes of actor / critic
-  int final_tanh;
-  float out_scale, clip_eps, ent_coef, inv_global_batch, rank_share;
+  float out_scale, ent_coef, rank_share;
   // outputs (nullable unless noted)
-  float* mean_out;           // [B, A]
-  float* value_out;          // [B]
   float* dz3_f32;            // [B, A]      dL/dz of the actor's output layer
   float* dv_f32;             // [B]         dL/dv
-  __nv_bfloat16* dz3_bf16;   // [B, dz3_pitch]
-  __nv_bfloat16* dv_bf16;    // [B, dv_pitch]
-  int dz3_pitch, dv_pitch;
   float* dz_a_f32;           // [B, hid_a]  dL/dz of the actor's last hidden layer
   float* dz_c_f32;           // [B, hid_c]
-  __nv_bfloat16* dz_a_bf16;  // [B, dz_a_pitch]
-  __nv_bfloat16* dz_c_bf16;
-  int dz_a_pitch, dz_c_pitch;
-  float* partials;           // [grid][2 + A] scratch (required)
-  unsigned* ticket;          // zero-initialised, self-resetting (required)
+  unsigned* ticket;          // zero-initialised, self-resetting (required; partials too)
   float* losses;             // [2]
   float* logstd_grad;        // [A]
 };

@@ -171,16 +171,24 @@ int cast_weights(b200ppo_ctx* ctx, const float* params, cudaStream_t st) {
   return launch_cast_weights(cast_group(ctx, params), st);
 }
 
-// forward of both nets on the tensor cores; hidden activations in bf16 (+ ones column), outputs in fp32.
-// The minibatch leaves the fused PPO epilogues of the output layers consume (nullptr = plain forward).
-struct PpoFuse {
-  const float *action, *old_logp, *advantage, *target;
-  const b200ppo_hparams* hp;
-  int loss_ctas;  // out: CTAs that wrote a row of loss partials
-};
+PpoOperands ppo_operands(const b200ppo_ctx* ctx, const float* params, const b200ppo_hparams* hp, int64_t B, const float* action,
+                         const float* old_logp, const float* adv, const float* tgt) {
+  PpoOperands op{};
+  op.logstd = params + ctx->logstd_off;
+  op.action = action; op.old_logp = old_logp; op.advantage = adv; op.target = tgt;
+  op.partials = ctx->loss_partials;
+  op.act_dim = ctx->net[0].out_dim();
+  op.final_tanh = ctx->net[0].d.final_tanh;
+  op.clip_eps = hp != nullptr ? float(hp->clip_epsilon) : 0.f;
+  op.inv_global_batch = 1.f / float(B * ctx->world);
+  return op;
+}
 
+// forward of both nets on the tensor cores; hidden activations in bf16 (+ ones column), outputs in fp32.
+// loss: the operands of the PPO loss fused into the output layers' epilogues (nullptr = plain forward); *loss_ctas is
+// then set to the number of CTAs that wrote a row of loss partials.
 static int forward_nets_bf16(b200ppo_ctx* ctx, const float* params, const __nv_bfloat16* xb, int64_t B,
-                             float* const outs[2], cudaStream_t st, PpoFuse* fuse = nullptr) {
+                             float* const outs[2], cudaStream_t st, const PpoOperands* loss = nullptr, int* loss_ctas = nullptr) {
   auto& bf = ctx->bf;
   const int maxL = max_layers(ctx, 3);
   for (int l = 0; l < maxL; ++l) {
@@ -201,18 +209,10 @@ static int forward_nets_bf16(b200ppo_ctx* ctx, const float* params, const __nv_b
       p.epilogue = TC_EPI_FWD;
       p.bias = params + N.b_off[l];
       p.bias_col = -1;
-      if (last && fuse != nullptr) {
+      if (last && loss != nullptr) {
         p.epilogue = n == 0 ? TC_EPI_PPO_ACTOR : TC_EPI_PPO_CRITIC;
         p.out_scale = N.d.out_scale;
-        p.ppo.logstd = params + ctx->logstd_off;
-        p.ppo.action = fuse->action; p.ppo.old_logp = fuse->old_logp; p.ppo.advantage = fuse->advantage;
-        p.ppo.target = fuse->target;
-        p.ppo.dz_out = bf.dZ[n][l]; p.ppo.dz_pitch = bf.pitchZ[n][l];
-        p.ppo.partials = ctx->loss_partials;
-        p.ppo.act_dim = ctx->net[0].out_dim();
-        p.ppo.final_tanh = N.d.final_tanh;
-        p.ppo.clip_eps = float(fuse->hp->clip_epsilon);
-        p.ppo.inv_global_batch = 1.f / float(B * ctx->world);
+        p.ppo = TcPpo{*loss, bf.dZ[n][l], bf.pitchZ[n][l]};
       } else if (last) {
         p.act = N.d.final_tanh ? TC_ACT_TANH_SCALE : TC_ACT_NONE;
         p.out_scale = N.d.out_scale;
@@ -228,7 +228,7 @@ static int forward_nets_bf16(b200ppo_ctx* ctx, const float* params, const __nv_b
     int grid = 0;
     // layer 0 may directly follow the optimizer (its weights are then one kernel old): only deeper layers preload W
     PROF(ctx, B200PPO_PROF_GEMM_FWD, st, ws ? launch_tc_ws(g, st, &grid, l > 0) : launch_tc_group(g, bn, st, &grid));
-    if (fuse != nullptr && l == maxL - 1) fuse->loss_ctas = grid;
+    if (loss != nullptr && l == maxL - 1) *loss_ctas = grid;
   }
   return B200PPO_OK;
 }
@@ -382,13 +382,7 @@ int launch_chain(b200ppo_ctx* ctx, const float* params, const __nv_bfloat16* xb,
     c.H1 = bf.H[n][0]; c.H2 = bf.H[n][1]; c.dZ1 = bf.dZ[n][0]; c.dZ2 = bf.dZ[n][1]; c.dZ3 = bf.dZ[n][2];
     c.pH1 = bf.pitchH[n][0]; c.pH2 = bf.pitchH[n][1]; c.pZ1 = bf.pitchZ[n][0]; c.pZ2 = bf.pitchZ[n][1]; c.pZ3 = bf.pitchZ[n][2];
   }
-  a.ppo.logstd = params + ctx->logstd_off;
-  a.ppo.action = action; a.ppo.old_logp = old_logp; a.ppo.advantage = adv; a.ppo.target = tgt;
-  a.ppo.partials = ctx->loss_partials;
-  a.ppo.act_dim = ctx->net[0].out_dim();
-  a.ppo.final_tanh = ctx->net[0].d.final_tanh;
-  a.ppo.clip_eps = hp != nullptr ? float(hp->clip_epsilon) : 0.f;
-  a.ppo.inv_global_batch = 1.f / float(B * ctx->world);
+  a.ppo = TcPpo{ppo_operands(ctx, params, hp, B, action, old_logp, adv, tgt)};
   if (inf != nullptr) {
     a.inf_noise = inf->noise; a.inf_mean = inf->mean; a.inf_value = inf->value; a.inf_action = inf->action; a.inf_logp = inf->logp;
     a.inf_ld_action = inf->ld_action > 0 ? inf->ld_action : ctx->net[0].out_dim();
@@ -405,19 +399,12 @@ int launch_chain(b200ppo_ctx* ctx, const float* params, const __nv_bfloat16* xb,
 }
 
 // the separate loss kernel's arguments: losses and the logstd gradient final, dL/dz of the output layers still to be set
-static LossArgs loss_args(const b200ppo_ctx* ctx, const float* params, float* const outs[2], const float* action,
-                          const float* old_logp, const float* adv, const float* tgt, int64_t B, const b200ppo_hparams* hp,
+static LossArgs loss_args(const b200ppo_ctx* ctx, const PpoOperands& op, float* const outs[2], int64_t B, const b200ppo_hparams* hp,
                           float* losses_dev) {
-  const Net& Na = ctx->net[0];
-  LossArgs la{};
-  la.mean = outs[0]; la.logstd = params + ctx->logstd_off; la.action = action; la.old_logp = old_logp;
-  la.advantage = adv; la.value = outs[1]; la.target = tgt; la.batch = B; la.act_dim = Na.out_dim();
-  la.final_tanh = Na.d.final_tanh; la.out_scale = Na.d.out_scale;
-  la.clip_eps = float(hp->clip_epsilon); la.ent_coef = float(hp->entropy_eps);
-  la.inv_global_batch = 1.f / float(B * ctx->world);
-  la.rank_share = 1.f / float(ctx->world);
-  la.partials = ctx->loss_partials; la.ticket = ctx->ticket;
-  la.losses = losses_dev; la.logstd_grad = ctx->gpart + ctx->logstd_off;
+  LossArgs la{op};
+  la.mean = outs[0]; la.value = outs[1]; la.batch = B; la.out_scale = ctx->net[0].d.out_scale;
+  la.ent_coef = float(hp->entropy_eps); la.rank_share = 1.f / float(ctx->world);
+  la.ticket = ctx->ticket; la.losses = losses_dev; la.logstd_grad = ctx->gpart + ctx->logstd_off;
   return la;
 }
 
@@ -431,6 +418,7 @@ int minibatch_fwd_bwd(b200ppo_ctx* ctx, const float* params, const float* obs, c
   const Net& Na = ctx->net[0];
   const Net& Nc = ctx->net[1];
   const int La = Na.d.n_layers, Lc = Nc.d.n_layers;
+  const PpoOperands op = ppo_operands(ctx, params, hp, B, action, old_logp, adv, tgt);
   if (ctx->precision == B200PPO_PREC_BF16) {
     // tcgen05 everywhere: forward (L launches; PPO loss fused into the output layers' epilogue), dgrads (L-1), wgrads (1)
     if (chain_applicable(ctx)) {  // one launch: forward, losses, dgrads (tc_chain.cu); then the weight gradients
@@ -442,13 +430,11 @@ int minibatch_fwd_bwd(b200ppo_ctx* ctx, const float* params, const float* obs, c
     const bool same_depth = La == Lc;  // both output layers in the same launch
     if (same_depth && tc_ppo_fits(Na.out_dim()) && Na.out_dim() <= 32 &&
         int64_t(2 * ((B + 127) / 128) + 8) <= ctx->loss_partial_rows) {
-      PpoFuse fuse{action, old_logp, adv, tgt, hp, 0};
-      B2_TRY(forward_nets_bf16(ctx, params, obs_b, B, outs, st, &fuse));
-      *loss_ctas_out = fuse.loss_ctas;
+      B2_TRY(forward_nets_bf16(ctx, params, obs_b, B, outs, st, &op, loss_ctas_out));
       return backward_nets_bf16(ctx, obs_b, B, ctx->gpart, split_out, st);
     }
     B2_TRY(forward_nets_bf16(ctx, params, obs_b, B, outs, st));
-    LossArgs la = loss_args(ctx, params, outs, action, old_logp, adv, tgt, B, hp, losses_dev);
+    LossArgs la = loss_args(ctx, op, outs, B, hp, losses_dev);
     la.dz_actor_bf16 = ctx->bf.dZ[0][La - 1]; la.dz_actor_pitch = ctx->bf.pitchZ[0][La - 1];
     la.dv_bf16 = ctx->bf.dZ[1][Lc - 1]; la.dv_pitch = ctx->bf.pitchZ[1][Lc - 1];
     PROF(ctx, B200PPO_PROF_LOSS, st, launch_ppo_loss(la, st));
@@ -458,24 +444,20 @@ int minibatch_fwd_bwd(b200ppo_ctx* ctx, const float* params, const float* obs, c
   SplitArena* arena = fresh_arena(ctx);
   PROF(ctx, B200PPO_PROF_GEMM_FWD, st, forward_nets(ctx, params, obs, B, 3, acts, outs, st, heads, arena));
   if (heads) {
-    HeadsArgs h{};
+    HeadsArgs h{op};
     h.h_a = acts[0] + Na.act_off(La - 2, B); h.h_c = acts[1] + Nc.act_off(Lc - 2, B);
     h.w3a = params + Na.w_off[La - 1]; h.b3a = params + Na.b_off[La - 1];
     h.w3c = params + Nc.w_off[Lc - 1]; h.b3c = params + Nc.b_off[Lc - 1];
-    h.logstd = params + ctx->logstd_off;
-    h.action = action; h.old_logp = old_logp; h.advantage = adv; h.target = tgt;
-    h.batch = B; h.act_dim = Na.out_dim(); h.hid_a = Na.d.dims[La - 2]; h.hid_c = Nc.d.dims[Lc - 2];
+    h.batch = B; h.hid_a = Na.d.dims[La - 2]; h.hid_c = Nc.d.dims[Lc - 2];
     h.act = Na.d.activation; h.act_c = Nc.d.activation;
-    h.final_tanh = Na.d.final_tanh; h.out_scale = Na.d.out_scale;
-    h.clip_eps = float(hp->clip_epsilon); h.ent_coef = float(hp->entropy_eps);
-    h.inv_global_batch = 1.f / float(B * ctx->world); h.rank_share = 1.f / float(ctx->world);
+    h.out_scale = Na.d.out_scale; h.ent_coef = float(hp->entropy_eps); h.rank_share = 1.f / float(ctx->world);
     h.dz3_f32 = dz[0] + Na.dz_off(La - 1, B); h.dv_f32 = dz[1] + Nc.dz_off(Lc - 1, B);
     h.dz_a_f32 = dz[0] + Na.dz_off(La - 2, B); h.dz_c_f32 = dz[1] + Nc.dz_off(Lc - 2, B);
-    h.partials = ctx->loss_partials; h.ticket = ctx->ticket;
+    h.ticket = ctx->ticket;
     h.losses = losses_dev; h.logstd_grad = ctx->gpart + ctx->logstd_off;
     PROF(ctx, B200PPO_PROF_LOSS, st, launch_heads(h, st));
   } else {
-    LossArgs la = loss_args(ctx, params, outs, action, old_logp, adv, tgt, B, hp, losses_dev);
+    LossArgs la = loss_args(ctx, op, outs, B, hp, losses_dev);
     la.dz_actor = dz[0] + Na.dz_off(La - 1, B);
     la.dv = dz[1] + Nc.dz_off(Lc - 1, B);
     PROF(ctx, B200PPO_PROF_LOSS, st, launch_ppo_loss(la, st));
@@ -485,14 +467,10 @@ int minibatch_fwd_bwd(b200ppo_ctx* ctx, const float* params, const float* obs, c
 
 LossCombine make_loss_combine(const b200ppo_ctx* ctx, const float* params, int loss_ctas, int64_t B, const b200ppo_hparams* hp,
                               float* losses_out) {
-  LossCombine lc{};
-  if (loss_ctas <= 0) return lc;
-  lc.partials = ctx->loss_partials;
+  if (loss_ctas <= 0) return LossCombine{};
+  LossCombine lc{ppo_operands(ctx, params, hp, B, nullptr, nullptr, nullptr, nullptr)};
   lc.n_cta = loss_ctas;
-  lc.act_dim = ctx->net[0].out_dim();
   lc.logstd_off = ctx->logstd_off;
-  lc.logstd = params + ctx->logstd_off;
-  lc.inv_global_batch = 1.f / float(B * ctx->world);
   lc.ent_coef = float(hp->entropy_eps);
   lc.rank_share = 1.f / float(ctx->world);
   lc.losses_out = losses_out;

@@ -1,8 +1,6 @@
-// Diagonal-Gaussian log-prob, entropy, clipped-ratio surrogate, Huber value loss and their gradient seeds.
-//
-// replaces: Normal.log_prob(...).sum(1), Normal.entropy().mean(), ratio/clamp/min/mean and huber_loss
-//           (src/entities/algorithms/ppo.py:113-132) together with what autograd derives from them
-//           (SURVEY.md §8a row a10), and Normal.sample / log_prob of the rollout (ppo.py:23-26).
+// Diagonal-Gaussian log-prob, entropy, clipped-ratio surrogate, Huber value loss and their gradient seeds (the math:
+// ppo_math.cuh) as a kernel of its own, for the shapes no fused route takes, and Normal.sample / log_prob of the
+// rollout (ppo.py:23-26).
 //
 // One thread per sample (rows are short: A floats).  Loss sums and the logstd gradient are reduced per CTA
 // in a fixed order and combined by the last CTA to finish (atomic ticket), so results are deterministic.
@@ -10,7 +8,6 @@
 
 namespace b200ppo {
 
-constexpr float kLogSqrt2Pi = 0.91893853320467274178f;  // math.log(math.sqrt(2*math.pi))
 constexpr int kLossThreads = 128;
 
 // One thread per sample row, but every global access is a block-wide contiguous slab copy: the 128 rows a CTA owns
@@ -32,17 +29,15 @@ ppo_loss_seed_kernel(LossArgs a) {
   __nv_bfloat16* s_dzb = reinterpret_cast<__nv_bfloat16*>(s_dl + kLossThreads * A);
   __shared__ float s_red[2][kLossThreads / 32];
   __shared__ float s_comb[kLossThreads];
-  __shared__ bool s_last;
   const int tid = threadIdx.x;
   const int64_t b0 = int64_t(blockIdx.x) * kLossThreads;
   const int64_t remaining = a.batch - b0;
   const int rows = remaining < kLossThreads ? int(remaining) : kLossThreads;
   for (int j = tid; j < A; j += kLossThreads) {
-    const float sig = expf(a.logstd[j]);
-    const float var = sig * sig;
-    s_logsig[j] = logf(sig);
-    s_inv_var[j] = 1.f / var;
-    s_two_var[j] = 2.f * var;
+    const PpoSigma c = ppo_sigma(a.logstd[j]);
+    s_logsig[j] = c.logsig;
+    s_inv_var[j] = c.inv_var;
+    s_two_var[j] = c.two_var;
   }
   for (int i = tid; i < rows * A; i += kLossThreads) {
     s_mean[i] = __ldg(a.mean + b0 * A + i);
@@ -58,53 +53,26 @@ ppo_loss_seed_kernel(LossArgs a) {
     const float* mu = s_mean + tid * A;
     const float* ac = s_act + tid * A;
     float lp = 0.f;
-    for (int j = 0; j < A; ++j) {
-      const float d = ac[j] - mu[j];
-      lp += -(d * d) / s_two_var[j] - s_logsig[j] - kLogSqrt2Pi;
-    }
+    for (int j = 0; j < A; ++j) lp += ppo_logp_term(ac[j] - mu[j], s_logsig[j], s_two_var[j]);
     if (a.logp_out != nullptr) a.logp_out[b] = lp;
     if (want_seed) {
-      const float adv = a.advantage[b];
-      const float ratio = expf(lp - a.old_logp[b]);
-      const float lo = 1.f - a.clip_eps, hi = 1.f + a.clip_eps;
-      const float s1 = ratio * adv;
-      const float s2 = fminf(fmaxf(ratio, lo), hi) * adv;
-      surr = fminf(s1, s2);
-      // autograd: minimum() sends the gradient to the smaller argument (half each on ties); clamp passes
-      // it inside [lo, hi] inclusive.
-      const float w1 = s1 < s2 ? 1.f : (s1 > s2 ? 0.f : 0.5f);
-      const float in_range = (ratio >= lo && ratio <= hi) ? 1.f : 0.f;
-      const float g_ratio = -(w1 * adv + (1.f - w1) * adv * in_range) * a.inv_global_batch;
-      const float g_lp = g_ratio * ratio;
+      const PpoSurrogate ps = ppo_surrogate(lp, a.old_logp[b], a.advantage[b], a.clip_eps, a.inv_global_batch);
+      surr = ps.surr;
       for (int j = 0; j < A; ++j) {
-        const float d = ac[j] - mu[j];
-        const float dn = d * s_inv_var[j];
-        float dmu = g_lp * dn;
-        if (a.final_tanh) {
-          const float th = mu[j] / a.out_scale;
-          dmu *= a.out_scale * (1.f - th * th);
-        }
+        const float d = ac[j] - mu[j], inv_var = s_inv_var[j];
+        const float dmu = ppo_mean_seed(ps.g_lp, d, inv_var, a.final_tanh, a.out_scale, [&] { return mu[j] / a.out_scale; });
         s_dz[tid * A + j] = dmu;
         if (a.dz_actor_bf16 != nullptr) s_dzb[tid * pitch + j] = __float2bfloat16_rn(dmu);
-        s_dl[tid * A + j] = g_lp * (d * dn - 1.f);
+        s_dl[tid * A + j] = ppo_logstd_term(ps.g_lp, d, inv_var);
       }
       if (a.dz_actor_bf16 != nullptr)
         for (int j = A; j < pitch; ++j) s_dzb[tid * pitch + j] = __float2bfloat16_rn(0.f);
     }
     if (a.dv != nullptr || a.dv_bf16 != nullptr) {
-      const float e = a.value[b] - a.target[b];
-      const float ae = fabsf(e);
-      hub = ae < 1.f ? 0.5f * e * e : ae - 0.5f;
-      const float dvv = fminf(fmaxf(e, -1.f), 1.f) * a.inv_global_batch;
-      if (a.dv != nullptr) a.dv[b] = dvv;
-      if (a.dv_bf16 != nullptr) {  // [B, dv_pitch] with the value in column 0: 16 bytes per row when dv_pitch == 8
-        if (a.dv_pitch == 8) {
-          const __nv_bfloat162 v0 = __floats2bfloat162_rn(dvv, 0.f);
-          *reinterpret_cast<uint4*>(a.dv_bf16 + b * 8) = make_uint4(*reinterpret_cast<const uint32_t*>(&v0), 0u, 0u, 0u);
-        } else {
-          for (int j = 0; j < a.dv_pitch; ++j) a.dv_bf16[b * a.dv_pitch + j] = __float2bfloat16_rn(j == 0 ? dvv : 0.f);
-        }
-      }
+      const PpoHuber h = ppo_huber(a.value[b], a.target[b], a.inv_global_batch);
+      hub = h.loss;
+      if (a.dv != nullptr) a.dv[b] = h.dv;
+      if (a.dv_bf16 != nullptr) ppo_store_dv_bf16(a.dv_bf16, b, a.dv_pitch, h.dv);
     }
   } else if (want_seed) {
     for (int j = 0; j < A; ++j) s_dl[tid * A + j] = 0.f;
@@ -138,29 +106,8 @@ ppo_loss_seed_kernel(LossArgs a) {
       part[2 + j] = s;
     }
   }
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) s_last = (atomicAdd(a.ticket, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  // last CTA: combine the per-CTA partials (fixed order, pipelined loads)
-  const float s = combine_partials<kLossThreads>(a.partials, gridDim.x, 2 + A, tid, s_comb);
-  const int c = tid;
-  if (c < 2 + A) {
-    if (c == 0) {
-      float ent = 0.f;  // mean over [B, A] of 0.5 + 0.5*log(2*pi) + log(sigma_j): the row is constant in b
-      for (int j = 0; j < A; ++j) ent += 0.5f + kLogSqrt2Pi + s_logsig[j];
-      ent /= float(A);
-      if (a.entropy_out != nullptr) *a.entropy_out = ent;
-      if (a.losses != nullptr) a.losses[0] = -s * a.inv_global_batch - a.ent_coef * ent * a.rank_share;
-    } else if (c == 1) {
-      if (a.losses != nullptr) a.losses[1] = s * a.inv_global_batch;
-    } else if (a.logstd_grad != nullptr) {
-      a.logstd_grad[c - 2] = s - a.ent_coef * a.rank_share / float(A);
-    }
-  }
-  if (tid == 0) *a.ticket = 0u;  // ready for the next launch on this stream
+  ppo_last_cta_finish<kLossThreads>(a, a.ent_coef, a.rank_share, a.ticket, s_comb, [&](int j) { return s_logsig[j]; }, a.losses,
+                                    a.logstd_grad, a.entropy_out);
 }
 
 __global__ void __launch_bounds__(128)
@@ -170,12 +117,11 @@ sample_logp_kernel(const float* __restrict__ mean, const float* __restrict__ log
   if (b >= batch) return;
   float lp = 0.f;
   for (int j = 0; j < A; ++j) {
-    const float sig = expf(__ldg(logstd + j));
+    const PpoSigma c = ppo_sigma(__ldg(logstd + j));
     const float mu = mean[b * A + j];
-    const float act = noise != nullptr ? mu + sig * noise[b * A + j] : mu;  // torch.normal(mean, std) = mean + std*eps
+    const float act = noise != nullptr ? mu + c.sig * noise[b * A + j] : mu;  // torch.normal(mean, std) = mean + std*eps
     if (action != nullptr) action[b * A + j] = act;
-    const float d = act - mu;
-    lp += -(d * d) / (2.f * (sig * sig)) - logf(sig) - kLogSqrt2Pi;
+    lp += ppo_logp_term(act - mu, c.logsig, c.two_var);
   }
   if (logp != nullptr) logp[b] = lp;
 }

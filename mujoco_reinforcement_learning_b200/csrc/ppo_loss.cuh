@@ -1,26 +1,16 @@
 // Internal interface of the loss / gradient-seed kernels (ppo_loss.cu).
 #pragma once
-#include <cuda_bf16.h>
-
-#include "common.cuh"
+#include "ppo_math.cuh"
 
 namespace b200ppo {
 
-struct LossArgs {
+struct LossArgs : PpoOperands {  // old_logp needed when dz_actor != null, target when dv != null
   // inputs
   const float* mean;       // [B, A] actor output (out_scale * tanh(z) when final_tanh)
-  const float* logstd;     // [A]
-  const float* action;     // [B, A]
-  const float* old_logp;   // [B]   (needed when dz_actor != null)
-  const float* advantage;  // [B]
   const float* value;      // [B]   critic output (needed when dv != null)
-  const float* target;     // [B]
   int64_t batch;           // local rows
-  int act_dim;
-  int final_tanh;
   float out_scale;
-  float clip_eps, ent_coef;
-  float inv_global_batch;  // 1 / (global minibatch size): the divisor of both loss means
+  float ent_coef;
   float rank_share;        // 1 / world_size: share of the batch-independent entropy term owned by this rank
   // outputs (all nullable)
   float* logp_out;      // [B] new log-prob
@@ -29,7 +19,6 @@ struct LossArgs {
   __nv_bfloat16* dz_actor_bf16;  // [B, dz_actor_pitch] bf16 copy for the tensor-core dgrad / wgrad (padding zeroed)
   __nv_bfloat16* dv_bf16;        // [B, dv_pitch]
   int dz_actor_pitch, dv_pitch;
-  float* partials;      // [grid][2 + A] scratch
   unsigned* ticket;     // zero-initialised counter, self-resetting
   float* losses;        // [2] actor_loss, critic_loss
   float* logstd_grad;   // [A]

@@ -469,8 +469,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
         b3_s[t] = t < A ? __ldg(a.net[0].b3 + t) : 0.f;
         float ls = 0.f, iv = 0.f;
         if (t < A) {
-          const float sig = expf(__ldg(a.ppo.logstd + t));
-          ls = logf(sig); iv = 1.f / (sig * sig);
+          const PpoSigma c = ppo_sigma(__ldg(a.ppo.logstd + t));
+          ls = c.logsig; iv = c.inv_var;
         }
         consts_s[t] = ls; consts_s[kChainMaxAct + t] = iv;
       } else if (t == kChainMaxAct) {
@@ -603,7 +603,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
                   const float nz = a.inf_noise != nullptr ? __ldg(a.inf_noise + mm * A + j) : 0.f;
                   if (a.inf_mean != nullptr) a.inf_mean[mm * A + j] = mean;
                   if (a.inf_action != nullptr) a.inf_action[mm * a.inf_ld_action + j] = mean + expf(consts_s[j]) * nz;
-                  lp += -0.5f * nz * nz - consts_s[j] - kTcLogSqrt2Pi;
+                  lp += -0.5f * nz * nz - consts_s[j] - kLogSqrt2Pi;
                 }
               }
             }
@@ -647,7 +647,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
               th[i] = ft ? tanh_fast(pre) : pre;
               const float mean = ft ? scale * th[i] : pre;
               d[i] = av[i] - mean;
-              lp += -(d[i] * d[i]) * (0.5f * consts_s[kChainMaxAct + j]) - consts_s[j] - kTcLogSqrt2Pi;
+              lp += ppo_logp_term_bf16(d[i], consts_s[j], consts_s[kChainMaxAct + j]);
             }
           }
         }
@@ -661,13 +661,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
         const float lp_row = ((l0 + l1) + l2) + l3;  // same order in all four warps
         float g_lp = 0.f, surr = 0.f;
         if (row_ok) {
-          const float lo = 1.f - a.ppo.clip_eps, hi = 1.f + a.ppo.clip_eps;
-          const float ratio = expf(lp_row - old_lp);
-          const float s1 = ratio * adv, s2 = fminf(fmaxf(ratio, lo), hi) * adv;
-          const float w1 = s1 < s2 ? 1.f : (s1 > s2 ? 0.f : 0.5f);
-          const float in_range = (ratio >= lo && ratio <= hi) ? 1.f : 0.f;
-          g_lp = -(w1 * adv + (1.f - w1) * adv * in_range) * a.ppo.inv_global_batch * ratio;
-          surr = fminf(s1, s2);
+          const PpoSurrogate ps = ppo_surrogate(lp_row, old_lp, adv, a.ppo.clip_eps, a.ppo.inv_global_batch);
+          g_lp = ps.g_lp;
+          surr = ps.surr;
         }
         uint32_t pk[4];
 #pragma unroll
@@ -678,11 +674,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
             const int j = j0 + i + u;
             dm[u] = 0.f;
             if (j < A) {
-              const float dn = d[i + u] * consts_s[kChainMaxAct + j];
-              float dmu = g_lp * dn;
-              if (ft) dmu *= scale * (1.f - th[i + u] * th[i + u]);
-              dm[u] = dmu;                              // g_lp = 0 for rows past the batch
-              d[i + u] = g_lp * (d[i + u] * dn - 1.f);  // this row's d loss / d logstd_j
+              dm[u] = ppo_mean_seed(g_lp, d[i + u], consts_s[kChainMaxAct + j], ft, scale, [&] { return th[i + u]; });  // g_lp = 0 for rows past the batch
+              d[i + u] = ppo_logstd_term(g_lp, d[i + u], consts_s[kChainMaxAct + j]);  // this row's d loss / d logstd_j
             }
           }
           pk[i >> 1] = pack_bf16(dm[0], dm[1]);
@@ -709,10 +702,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1) tc_ch
           tmem_ld8(lane_base + 256u, v);
           float dv = 0.f, hub = 0.f;
           if (row_ok) {
-            const float e = __uint_as_float(v[0]) + b3_s[kChainMaxAct] - tgt;
-            const float ae = fabsf(e);
-            hub = ae < 1.f ? 0.5f * e * e : ae - 0.5f;
-            dv = fminf(fmaxf(e, -1.f), 1.f) * a.ppo.inv_global_batch;
+            const PpoHuber h = ppo_huber(__uint_as_float(v[0]) + b3_s[kChainMaxAct], tgt, a.ppo.inv_global_batch);
+            hub = h.loss;
+            dv = h.dv;
           }
           const uint32_t w0 = pack_bf16(dv, 0.f);
           asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(row_z3c + ((0u ^ sw) << 4)), "r"(w0), "r"(0u), "r"(0u), "r"(0u) : "memory");

@@ -508,8 +508,7 @@ inline bool tc_can_stage(const TcProblem& p) {
   return false;
 }
 
-// ---- fused PPO-loss epilogues of the output layers ---------------------------------------------------------------------
-constexpr float kTcLogSqrt2Pi = 0.91893853320467274178f;
+// ---- fused PPO-loss epilogues of the output layers (the math: ppo_math.cuh) ---------------------------------------------
 
 struct PpoAcc {  // per-thread running sums over the tiles a CTA processes
   float surr, hub;
@@ -527,9 +526,8 @@ __device__ __forceinline__ void tc_ppo_stage_consts(const TcProblem& P, float* c
   if (P.epilogue == TC_EPI_PPO_ACTOR && tid < 32) {
     float ls = 0.f, iv = 0.f, tv = 1.f;
     if (tid < P.ppo.act_dim) {
-      const float sig = expf(__ldg(P.ppo.logstd + tid));
-      const float var = sig * sig;
-      ls = logf(sig); iv = 1.f / var; tv = 2.f * var;
+      const PpoSigma c = ppo_sigma(__ldg(P.ppo.logstd + tid));
+      ls = c.logsig; iv = c.inv_var; tv = c.two_var;
     }
     consts_s[tid] = ls; consts_s[32 + tid] = iv; consts_s[64 + tid] = tv;
   }
@@ -589,19 +587,15 @@ __device__ __forceinline__ void tc_ppo_actor_row(const TcProblem& P, uint32_t tm
       const float th = ft ? tanh_fast(pre) : pre;
       const float mean = ft ? scale * th : pre;
       const float d = act_s[j] - mean;
-      lp += -(d * d) * (0.5f * consts_s[32 + j]) - consts_s[j] - kTcLogSqrt2Pi;  // -(a-mu)^2 / (2 var) - log sigma - log sqrt(2 pi)
+      lp += ppo_logp_term_bf16(d, consts_s[j], consts_s[32 + j]);
       z[j] = d;  // keep (a - mean); tanh is recovered below as (a - d) / scale
     }
   }
   float g_lp = 0.f;
   if (row_ok) {
-    const float lo = 1.f - P.ppo.clip_eps, hi = 1.f + P.ppo.clip_eps;
-    const float ratio = expf(lp - old_lp);
-    const float s1 = ratio * adv, s2 = fminf(fmaxf(ratio, lo), hi) * adv;
-    const float w1 = s1 < s2 ? 1.f : (s1 > s2 ? 0.f : 0.5f);
-    const float in_range = (ratio >= lo && ratio <= hi) ? 1.f : 0.f;
-    g_lp = -(w1 * adv + (1.f - w1) * adv * in_range) * P.ppo.inv_global_batch * ratio;
-    acc.surr += fminf(s1, s2);
+    const PpoSurrogate ps = ppo_surrogate(lp, old_lp, adv, P.ppo.clip_eps, P.ppo.inv_global_batch);
+    g_lp = ps.g_lp;
+    acc.surr += ps.surr;
   }
   uint32_t packed[NC / 2];
 #pragma unroll
@@ -613,14 +607,9 @@ __device__ __forceinline__ void tc_ppo_actor_row(const TcProblem& P, uint32_t tm
       dm[u] = 0.f;
       if (jj < A) {
         const float d = z[jj];
-        const float dn = d * consts_s[32 + jj];
-        float dmu = g_lp * dn;
-        if (ft) {
-          const float th = (act_s[jj] - d) * inv_scale;  // mean / scale
-          dmu *= scale * (1.f - th * th);
-        }
+        const float dmu = ppo_mean_seed(g_lp, d, consts_s[32 + jj], ft, scale, [&] { return (act_s[jj] - d) * inv_scale; });  // mean / scale
         dm[u] = row_ok ? dmu : 0.f;
-        if (row_ok) acc.dl[jj] += g_lp * (d * dn - 1.f);
+        if (row_ok) acc.dl[jj] += ppo_logstd_term(g_lp, d, consts_s[32 + jj]);
       }
     }
     packed[j >> 1] = pack_bf16(dm[0], dm[1]);
@@ -660,19 +649,9 @@ __device__ __forceinline__ void tc_epilogue_ppo(const TcProblem& P, uint32_t tme
     uint32_t v[16];
     tmem_ld16(tmem_acc + (uint32_t(q * 32) << 16), v);
     if (row_ok) {
-      const float val = __uint_as_float(v[0]) + bias_s[0];
-      const float e = val - tgt;
-      const float ae = fabsf(e);
-      acc.hub += ae < 1.f ? 0.5f * e * e : ae - 0.5f;
-      const float dv = fminf(fmaxf(e, -1.f), 1.f) * P.ppo.inv_global_batch;
-      const int pitch = P.ppo.dz_pitch;
-      __nv_bfloat16* o = P.ppo.dz_out + int64_t(m) * pitch;
-      if (pitch == 8) {
-        const __nv_bfloat162 v0 = __floats2bfloat162_rn(dv, 0.f);
-        *reinterpret_cast<uint4*>(o) = make_uint4(*reinterpret_cast<const uint32_t*>(&v0), 0u, 0u, 0u);
-      } else {
-        for (int j = 0; j < pitch; ++j) o[j] = __float2bfloat16_rn(j == 0 ? dv : 0.f);
-      }
+      const PpoHuber h = ppo_huber(__uint_as_float(v[0]) + bias_s[0], tgt, P.ppo.inv_global_batch);
+      acc.hub += h.loss;
+      ppo_store_dv_bf16(P.ppo.dz_out, m, P.ppo.dz_pitch, h.dv);
     }
     return;
   }

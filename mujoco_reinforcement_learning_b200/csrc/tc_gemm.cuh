@@ -5,6 +5,7 @@
 #include <string.h>
 
 #include "common.cuh"
+#include "ppo_math.cuh"
 
 namespace b200ppo {
 
@@ -19,16 +20,9 @@ enum TcEpilogue : int {
 };
 
 // Extra operands of the fused PPO epilogues (src/entities/algorithms/ppo.py:113-132).
-struct TcPpo {
-  const float* logstd;     // [A]
-  const float* action;     // [M, A]
-  const float* old_logp;   // [M]
-  const float* advantage;  // [M]
-  const float* target;     // [M]
+struct TcPpo : PpoOperands {
   __nv_bfloat16* dz_out;   // actor: [M, dz_pitch] ; critic: [M, dz_pitch] with dv in column 0
-  float* partials;         // [gridDim.x][2 + A]: (sum surrogate, sum huber, sum d loss / d logstd_j) per CTA
-  int dz_pitch, act_dim, final_tanh;
-  float clip_eps, inv_global_batch;
+  int dz_pitch;
 };
 
 // activation codes of TC_EPI_FWD beyond B200PPO_ACT_TANH / B200PPO_ACT_RELU

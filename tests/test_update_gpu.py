@@ -173,7 +173,9 @@ def test_train_matches_reference_outputs(name):
                                    dict(D=27, A=8, H=[256, 256], N=32, T=32, B=256),      # Ant dims
                                    dict(D=376, A=17, H=[256, 256], N=64, T=128, B=4096),  # fp32-tolerance GEMMs on the tensor cores
                                    dict(D=11, A=3, H=[64, 64], N=16, T=256, B=4096),      # Hopper config, one big batch
-                                   dict(D=17, A=6, H=[64, 64], N=1, T=2048, B=500)])      # HalfCheetah config
+                                   dict(D=17, A=6, H=[64, 64], N=1, T=2048, B=500),       # HalfCheetah config
+                                   # last hidden width not a multiple of 4: the separate loss kernel's fp32 seeds
+                                   dict(D=11, A=3, H=[30, 18], N=16, T=64, B=512)])
 def test_train_vs_oracle_on_baseline_shapes(shape):
     _train_vs_oracle(shape, terms=3)
 
@@ -281,6 +283,8 @@ def test_bf16_minibatch_losses_and_gradients_vs_oracle(name):
                                    dict(D=376, A=17, H=[256, 256], N=16, T=64, B=500),
                                    dict(D=27, A=8, H=[256, 256], N=32, T=32, B=256),
                                    dict(D=11, A=3, H=[64, 64], N=16, T=256, B=1024),
+                                   # enough row tiles for the persistent kernel: the PPO loss in tc_ws_kernel's epilogue
+                                   dict(D=11, A=3, H=[64, 64], N=64, T=640, B=20480),
                                    # the bench minibatch: CTA-pair forward / dgrad / wgrad kernels, fused-loss output layer
                                    dict(D=376, A=17, H=[256, 256], N=256, T=128, B=32768)])
 def test_bf16_train_vs_oracle(shape):
